@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — UAV env-steps/s of the batched environment step on B200, next to the reference CPU step.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c4s|...] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c4s|...] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (one `uavca_step_*` launch) over one batch of B envs.  Default workload:
 BASELINE.json configs[2] at N=1 GPU — multi-UAV, N=8 UAVs per env, B=65,536 envs, random cartesian actions, auto-reset
@@ -57,6 +57,7 @@ WORKLOADS = {
 L2_BYTES = 126e6
 GRAPH_STEPS = 200
 MIN_REPS, MAX_REPS, LOADED_MS = 5, 400, 60.0  # repetitions of the K-step region; enough of them to sample clocks under load
+DUMP_BYTES = 60_000_000  # --dump-outputs writes at most this much (plus .npy headers), under 64 MB
 
 
 def algorithmic_bytes_per_unit(kind: str, N: int) -> float:
@@ -459,6 +460,14 @@ def run_ours(args, wl, rank, world, local_rank):
         del keepS
     else:
         tS, clocks = t1, clocks1
+    dump = args.dump_outputs if rank == 0 else None
+    per_step_out = None
+    if dump:  # the batch that took the last step of the timed graphs (graphs_for: steps W .. W+199, then the remainder)
+        e = envs[(W + GRAPH_STEPS - 1 + K % GRAPH_STEPS) % ring]
+        last = dict(obs=e.obs, reward=e.reward, done=e.done)
+        if kind == "single":
+            last["distance"] = e.distance
+        per_step_out = output_sample(last)
 
     def reduce_reps(ts):
         ts = [sharding.max_over_ranks(t, device=dev) for t in ts] if dist is not None else ts
@@ -470,19 +479,23 @@ def run_ours(args, wl, rank, world, local_rank):
     per_step_value = world * units_per_step * K / (ms_med * 1e-3)
 
     # ---- K steps per launch (uavca_rollout), ONE stream: an action block resident in HBM, and on-device Philox actions
-    rollout = None
+    rollout = rollout_out = None
     if not args.no_rollout:
         rollout = measure_rollout(torch, G, envs, ring, kind, N, B, amax, dev, stream, barrier, reduce_reps, world, args.rollout_k, K,
-                                  local_rank)
+                                  local_rank, keep_last=dump is not None)
         if rollout is not None:
             gpu_launches += rollout.pop("_launches")
+            rollout_out = rollout.pop("_last", None)
     headline_rollout = rollout is not None and args.headline == "rollout"
+    if dump:
+        write_outputs(dump, rollout_out if headline_rollout else per_step_out)
 
     # ---- BASELINE configs[4] beside it (one GPU, default workload only): policy + env step + replay append per acting step
     acting = None
     if world == 1 and args.workload == "c3" and not args.no_acting:
         a_wl = WORKLOADS["c5r"]
-        rows, a_launches = measure_acting(args, G, torch, dev, rank, world, dist, barrier, a_wl["B"], a_wl["N"], min(K, 400))
+        rows, a_launches, _ = measure_acting(args, G, torch, dev, rank, world, dist, barrier, a_wl["B"], a_wl["N"],
+                                             max(2, min(K, 400) // 2 * 2))
         acting = {"workload": a_wl["desc"], "rows": rows,
                   "what": "us per acting step and UAV env-steps/s; fp32 = eager PyTorch policy in the reference's arithmetic, "
                           "fused = uavca_policy_act (one tcgen05 kernel, fp16 operands / fp32 accumulate)"}
@@ -709,11 +722,13 @@ def measure_pcie(torch, dev, env, h_obs, h_act, d_act, barrier, sharding):
         return {"unavailable": repr(exc)[:160]}
 
 
-def measure_rollout(torch, G, envs, ring, kind, N, B, amax, dev, stream, barrier, reduce_reps, world, Kr, K, local_rank):
+def measure_rollout(torch, G, envs, ring, kind, N, B, amax, dev, stream, barrier, reduce_reps, world, Kr, K, local_rank,
+                    keep_last=False):
     """`uavca_rollout` on ONE stream: a repetition is exactly K env steps, done as launches of Kr steps (+ one launch of
     the remainder), each launch on the next batch of the ring (every launch finds its state in HBM, not in L2); the
     [Kr, ...] output blocks (>> L2) are shared by the batches.  Two variants: actions from an action block resident in
-    HBM, and on-device Philox actions (the run_multi.py loop)."""
+    HBM, and on-device Philox actions (the run_multi.py loop).  `keep_last`: `_last` holds the `output_sample` of the
+    last step of the action-block variant."""
     M = B * N
     if kind != "single" and (M * 10 * 4) % 16:
         return None
@@ -736,9 +751,11 @@ def measure_rollout(torch, G, envs, ring, kind, N, B, amax, dev, stream, barrier
                 k = Kr if i < q else rem
                 j = state["j"]
                 acts = None if name == "philox" else blocks[j % n_blocks][:k]
-                envs[j % ring].rollout(k, acts, action_seed=1, step0=state["t"], out=(outs if i < q else outs_rem)[j % 2], sync_last=False)
+                o = (outs if i < q else outs_rem)[j % 2]
+                envs[j % ring].rollout(k, acts, action_seed=1, step0=state["t"], out=o, sync_last=False)
                 state["t"] += k
                 state["j"] = j + 1
+                state["last"] = (o, k)
 
         with torch.cuda.stream(stream):
             rep()
@@ -746,6 +763,9 @@ def measure_rollout(torch, G, envs, ring, kind, N, B, amax, dev, stream, barrier
         est_ms = K * M * 45 / 3.0e12 * 1e3
         with ClockSampler(local_rank) as clocks:
             ts = timed_reps(torch, stream, rep, est_ms, dev, barrier)
+        if keep_last and name == "block":
+            o, k = state["last"]
+            res["_last"] = output_sample({key: v[k - 1] for key, v in o.items()})
         med, best, n = reduce_reps(ts)
         us_per_step = med * 1e3 / K
         moved = rollout_bytes_per_unit(kind, N, name == "block")
@@ -780,12 +800,15 @@ def run_c1(args, wl, G, torch, dev):
         l0 = env._b.launch_count
         t0 = time.perf_counter()
         for a in acts:
-            _, _, done, _ = env.step(a)
+            obs, reward, done, info = env.step(a)
             if done:
                 env.reset()
         dt = time.perf_counter() - t0
         launches = env._b.launch_count - l0
         best = dt if best is None else min(best, dt)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, output_sample(dict(obs=obs[None], reward=np.array([reward]), done=np.array([done], np.float32),
+                                                            distance=np.array([info["distance"]]))))
     lit = literal_baseline("single", 1) if not args.no_cpu_baseline else None
     emit({"metric": "UAV env-steps/sec", "value": K / best, "unit": "UAV env-steps/s", "n_gpus": 1, "steps": K, "warmup": args.warmup,
           "ms_per_step": best / K * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -796,10 +819,12 @@ def run_c1(args, wl, G, torch, dev):
           "gpu_launches": int(launches), "roofline": None, "cpu_baseline": lit, "cpu_baseline_literal": lit})
 
 
-def measure_acting(args, G, torch, dev, rank, world, dist, barrier, B, N, K):
+def measure_acting(args, G, torch, dev, rank, world, dist, barrier, B, N, K, keep_row=None):
     """BASELINE configs[4]: one acting step = policy forward over all B*N observations + env step (polar action map
     fused) + append of the B*N transitions to the device replay ring.  Rows: eager fp32 (the reference's arithmetic),
-    TF32, and the fused tcgen05 acting kernel.  Returns (rows, launches of ours)."""
+    TF32, and the fused tcgen05 acting kernel.  A repetition is K acting steps (K even: the rollout ping-pongs two
+    observation buffers, so every CUDA graph holds an even number of steps).  Returns (rows, launches of ours, the
+    `output_sample` of the last step of row `keep_row` or None)."""
     from gym_uav_collision_avoidance_b200 import sharding
 
     torch.manual_seed(0)
@@ -808,6 +833,7 @@ def measure_acting(args, G, torch, dev, rank, world, dist, barrier, B, N, K):
     rows = {}
     stream = torch.cuda.Stream(device=dev)
     total_launches = 0
+    kept = None
     for row in ("fp32", "tf32", "fused", "fused_separate_append"):
         precision = "fused" if row.startswith("fused") else row
         env = G.BatchedMultiUAVWorld2D(B, num_agents=N, reset_mode=G.RESET_ON_DONE0, max_episode_steps=1500, seed=0x5EED,
@@ -824,32 +850,41 @@ def measure_acting(args, G, torch, dev, rank, world, dist, barrier, B, N, K):
             for _ in range(3):
                 ro.step()
         torch.cuda.synchronize(dev)
-        n_graph = max(2, min(K, 50) // 2 * 2)  # even: the rollout ping-pongs two observation buffers
-        g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g, stream=stream):
-            for _ in range(n_graph):
-                ro.step()
-        g.replay()
-        torch.cuda.synchronize(dev)
-        q = max(1, K // n_graph)
+        n_graph = min(K, 50)
+        q, rem = divmod(K, n_graph)
 
-        def rep(g=g, q=q):
+        def capture(n):
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g, stream=stream):
+                for _ in range(n):
+                    ro.step()
+            g.replay()
+            return g
+
+        g, g_rem = capture(n_graph), capture(rem) if rem else None
+        torch.cuda.synchronize(dev)
+
+        def rep(g=g, q=q, g_rem=g_rem):
             for _ in range(q):
                 g.replay()
+            if g_rem is not None:
+                g_rem.replay()
 
-        ts = timed_reps(torch, stream, rep, (0.07 if precision == "fused" else 1.0) * q * n_graph, dev, barrier)
+        ts = timed_reps(torch, stream, rep, (0.07 if precision == "fused" else 1.0) * K, dev, barrier)
         ts = [sharding.max_over_ranks(t, device=dev) for t in ts] if dist is not None else ts
+        if row == keep_row:
+            kept = output_sample(dict(obs=env.obs, reward=env.reward, done=env.done, action=ro.action))
         med = statistics.median(ts)
-        us = med * 1e3 / (q * n_graph)
-        rows[row] = {"us_per_acting_step": us, "value": world * B * N / us * 1e6, "best_us": min(ts) * 1e3 / (q * n_graph),
-                     "repetitions": len(ts), "steps_per_repetition": q * n_graph, "replay_size": len(replay),
+        us = med * 1e3 / K
+        rows[row] = {"us_per_acting_step": us, "value": world * B * N / us * 1e6, "best_us": min(ts) * 1e3 / K,
+                     "repetitions": len(ts), "steps_per_repetition": K, "replay_size": len(replay),
                      "launches_per_acting_step": (2 if ro.fused_append else 3) if precision == "fused" else None}
         if head_err is not None:
             rows[row]["head_max_abs_err_vs_fp64"] = head_err
         total_launches += env.launch_count
-        del g, ro, replay, env
+        del g, g_rem, ro, replay, env
     torch.backends.cuda.matmul.allow_tf32 = tf32_before
-    return rows, total_launches
+    return rows, total_launches, kept
 
 
 def policy_head_error(G, torch, policy, ro, env):
@@ -876,8 +911,11 @@ def policy_head_error(G, torch, policy, ro, env):
 def run_acting(args, wl, G, torch, dev, rank, world, dist, barrier):
     """`--workload c5r`: the acting step as the headline; value = the fp32 row unless --acting-precision says otherwise."""
     B, N, K = wl["B"], wl["N"], args.steps
-    rows, total_launches = measure_acting(args, G, torch, dev, rank, world, dist, barrier, B, N, K)
     head = args.acting_precision
+    rows, total_launches, last = measure_acting(args, G, torch, dev, rank, world, dist, barrier, B, N, K,
+                                                keep_row=head if args.dump_outputs and rank == 0 else None)
+    if last is not None:
+        write_outputs(args.dump_outputs, last)
     if rank == 0:
         us = rows[head]["us_per_acting_step"]
         emit({"metric": "UAV env-steps/sec", "value": rows[head]["value"], "unit": "UAV env-steps/s", "n_gpus": world, "steps": K,
@@ -910,6 +948,37 @@ def emit(line: dict):
     out.flush()
 
 
+def output_sample(arrays: dict, seed: int = 0) -> dict:
+    """Host copies of the outputs a caller of the timed path received in its last step (`arrays`: name -> tensor or array
+    whose axis 0 is the env axis), as float32 (float64 and int64 as float64).  Where all of them together exceed
+    DUMP_BYTES, the same envs of every array are kept: a sorted sample drawn with `seed`, so that runs with the same
+    arguments keep the same envs.  `env_index` lists the envs kept (indices into the batch)."""
+    import numpy as np
+    import torch
+
+    ts = {k: torch.as_tensor(v) for k, v in arrays.items()}
+    wide = (torch.float64, torch.int64)
+    n = next(iter(ts.values())).shape[0]
+    per_env = 8 + sum(t[:1].numel() * (8 if t.dtype in wide else 4) for t in ts.values())
+    keep = min(n, DUMP_BYTES // per_env)
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+    out = {}
+    for k, t in ts.items():
+        sel = t[torch.as_tensor(idx, device=t.device)] if keep < n else t
+        out[k] = sel.to(torch.float64 if t.dtype in wide else torch.float32).cpu().numpy()
+    out["env_index"] = idx.astype(np.float64)
+    return out
+
+
+def write_outputs(path: str, sample: dict):
+    """--dump-outputs: one DIR/<name>.npy per array of `output_sample`."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    for k, a in sample.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -929,11 +998,21 @@ def main():
     ap.add_argument("--acting-precision", default="fp32", choices=["fp32", "tf32", "fused"])
     ap.add_argument("--streams", type=int, default=None,
                     help="streams the independent batches of the ring are pipelined over (default: 2; 4 for the small c2/c5 batches)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the headline path returned in its last step as DIR/<name>.npy "
+                         "(float32 / float64, at most 64 MB: a fixed sample of envs where the batch is larger; rank 0's "
+                         "shard); inputs are seeded, so runs with the same arguments can be compared file by file")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the outputs of --impl ours")
     protect_stdout()
     if args.workload is None:
         args.workload = "c3" if args.gpus <= 1 else "c4s"
     wl = WORKLOADS[args.workload]
+    if args.workload == "c5r" and args.steps is not None and args.steps % 2:
+        ap.error("--workload c5r times an even number of steps (the acting step alternates two observation buffers)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -3,6 +3,7 @@
 Run in the build container (where /root/reference exists):
 
     python -m oracle.gen_golden            # rewrites tests/golden/*.npz
+    python -m oracle.gen_golden live       # rewrites tests/golden/live_reference_digests.json (oracle only)
 
 Every file holds seeded initial states, the float32 actions that were fed (to the reference as float64
 up-casts, SURVEY.md §8c), and what the literal reference returned at every step: float64 observations and
@@ -76,11 +77,9 @@ def _actions_multi_f64(rng, st: O.State, b: int, N: int, controller: bool):
     return np.stack([v * np.cos(th), v * np.sin(th)], axis=1).astype(np.float64)
 
 
-def run_reference_multi(case) -> dict:
-    _, MultiUAVWorld2D = R.load_reference()
-    N, E, T = case["N"], case["E"], case["T"]
-    rng = np.random.default_rng(case["seed"])
-    # odd envs: crowded region + controller; even envs: full box + random actions
+def _init_and_pool(case, rng):
+    """Seeded initial states and reset pool of a multi case: odd envs in a crowded region, even envs in the full box."""
+    N, E = case["N"], case["E"]
     regions = [None if b % 2 == 0 else max(3.0, 0.75 * N ** 0.5 * 2.0) for b in range(E)]
     init = O.State(E, N)
     for b in range(E):
@@ -92,6 +91,15 @@ def run_reference_multi(case) -> dict:
         s = O.sample_multi_states(1, N, rng, region=regions[p % E])
         for f in ("pos", "vel", "tgt", "init", "prev", "flags"):
             getattr(pool, f)[p] = getattr(s, f)[0]
+    return init, pool
+
+
+def run_reference_multi(case) -> dict:
+    _, MultiUAVWorld2D = R.load_reference()
+    N, E, T = case["N"], case["E"], case["T"]
+    rng = np.random.default_rng(case["seed"])
+    # odd envs: crowded region + controller; even envs: full box + random actions
+    init, pool = _init_and_pool(case, rng)
 
     envs = [MultiUAVWorld2D(num_agents=N) for _ in range(E)]
     cur = init.copy()
@@ -252,11 +260,114 @@ def run_reference_single(case) -> dict:
     return res
 
 
+# ---- the live checks of tests/test_oracle_golden.py, kept runnable without the reference ---------------------------
+# Their inputs come from seeded NumPy generators and from the state of the world being stepped, never from the reference
+# itself, so the oracle regenerates them exactly.  LIVE_DIGESTS stores, per step, a digest of the exact bytes of those
+# inputs and of everything the checks compare; where the reference is present the tests still compare it live as well.
+LIVE_DIGESTS = os.path.join(GOLDEN_DIR, "live_reference_digests.json")
+LIVE_MULTI_N = (3, 7)
+RANDOM_WORLD_TRIALS = 6
+
+
+def digest(*arrays) -> str:
+    """First 128 bits of SHA-256 over the exact bytes of `arrays` (None skipped)."""
+    import hashlib
+
+    h = hashlib.sha256()
+    for a in arrays:
+        if a is not None:
+            h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()[:32]
+
+
+def live_multi_case(n: int) -> dict:
+    return dict(name="live", N=n, E=4, T=120, seed=900 + n, evaluate=0, reset_mode=O.RESET_ON_DONE0, max_steps=60)
+
+
+def oracle_live_multi(case):
+    """The oracle's side of run_reference_multi(case): the same initial states, pool and action draws (made from the
+    oracle's state, which is the reference's as long as the two agree).  Yields (action, step outputs, state) per step."""
+    N, E = case["N"], case["E"]
+    rng = np.random.default_rng(case["seed"])
+    init, pool = _init_and_pool(case, rng)
+    orc = O.Oracle(O.multi_config(E, N, reset_mode=case["reset_mode"], max_episode_steps=case["max_steps"],
+                                  reset_source=O.SOURCE_POOL))
+    for f in ("pos", "vel", "tgt", "init", "prev", "flags"):
+        getattr(orc.state, f)[...] = getattr(init, f)
+    orc.state.episode[...] = 1
+    orc.set_pool(pool)
+    for _ in range(case["T"]):
+        a = np.stack([_actions_multi(rng, orc.state, b, N, controller=(b % 2 == 1)) for b in range(E)])
+        yield a, orc.step(a, evaluate=bool(case["evaluate"]), want_final_obs=True), orc.state
+
+
+def live_multi_digest(a, out, st) -> str:
+    return digest(a, out["done"], out["reset_mask"], out["reward"], out["obs"], out["final_obs"], st.pos, st.vel)
+
+
+def oracle_random_world(trial: int):
+    """A non-default world drawn at random (box, speed / acceleration bounds, collider radius, sensing range, N), crowded
+    enough for collisions, goal reaches and parked UAVs, stepped 250 times by the oracle.  Yields first the setup
+    dict(n, kw, state, obs0, evaluate, f64), then (action, step outputs, state) per step; half of the trials feed float64
+    actions that float32 cannot hold."""
+    rng = np.random.default_rng(4100 + trial)
+    n = int(rng.choice([2, 3, 6, 9, 12, 17]))
+    kw = dict(x_size=float(rng.uniform(10, 40)), y_size=float(rng.uniform(10, 40)), max_speed=float(rng.uniform(3, 20)),
+              max_acceleration=float(rng.uniform(1, 12)), collider_radius=float(rng.uniform(0.3, 1.5)),
+              d_sense=float(rng.choice([rng.uniform(1.0, 4.0), rng.uniform(6, 40)])))
+    st = O.sample_multi_states(1, n, rng, x_size=kw["x_size"], y_size=kw["y_size"], collider_radius=kw["collider_radius"],
+                               region=min(kw["x_size"], kw["y_size"]) / 3)
+    orc = O.Oracle(O.multi_config(1, n, **kw))
+    orc.state = st.copy()
+    evaluate, f64 = bool(trial % 2), trial >= 3
+    yield dict(n=n, kw=kw, state=st, obs0=orc.observe()[0], evaluate=evaluate, f64=f64)
+    for t in range(250):
+        if t % 3:
+            a = np.clip((orc.state.tgt[0] - orc.state.pos[0]) * 1.2 + rng.normal(0, 0.4, (n, 2)), -kw["max_speed"], kw["max_speed"])
+        else:
+            a = rng.uniform(-kw["max_speed"], kw["max_speed"], (n, 2))
+        a = a.astype(np.float64) if f64 else a.astype(np.float32)
+        out = orc.step_f64(a[None], evaluate=evaluate) if f64 else orc.step(a[None], evaluate=evaluate)
+        yield a, out, orc.state
+
+
+def random_world_setup_digest(setup) -> str:
+    st = setup["state"]
+    return digest(np.array(json.dumps(setup["kw"], sort_keys=True)), st.pos, st.vel, st.tgt, st.init, st.prev, st.flags, setup["obs0"])
+
+
+def random_world_digest(a, out, st) -> str:
+    return digest(a, out["done"], out["reward"], out["obs"], st.pos, st.vel, st.prev, st.flags, st.coll, st.reach)
+
+
+def record_live_digests() -> str:
+    """Write LIVE_DIGESTS from the oracle (`python -m oracle.gen_golden live`)."""
+    rec = {"about": "Per-step digests (first 128 bits of SHA-256 over the exact bytes) of oracle/uav_oracle.c on the inputs of "
+                     "the live checks in tests/test_oracle_golden.py, recorded by `python -m oracle.gen_golden live`.  Those "
+                     "checks demand exact equality with the reference at every step; where the reference is present they "
+                     "still run it live beside these digests.",
+           "live_multi": {}, "random_world": {}}
+    for n in LIVE_MULTI_N:
+        rec["live_multi"][str(n)] = [live_multi_digest(*s) for s in oracle_live_multi(live_multi_case(n))]
+    for trial in range(RANDOM_WORLD_TRIALS):
+        gen = oracle_random_world(trial)
+        setup = next(gen)
+        rec["random_world"][str(trial)] = {"n": setup["n"], "kw": setup["kw"], "setup": random_world_setup_digest(setup),
+                                           "steps": [random_world_digest(*s) for s in gen]}
+    with open(LIVE_DIGESTS, "w") as f:
+        json.dump(rec, f, indent=0)
+        f.write("\n")
+    return LIVE_DIGESTS
+
+
 def main():
     import sys
 
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     only = sys.argv[1] if len(sys.argv) > 1 else None  # "circular" or a case name: regenerate just those cases
+    if only == "live":
+        print(record_live_digests())
+        return
     if only and only not in ("circular", "f64act"):
         for case in MULTI_CASES:
             if case["name"] == only:

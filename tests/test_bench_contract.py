@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -60,3 +63,52 @@ def test_multi_gpu_default_workload_is_configs3():
     d = json.loads(out.stdout.strip().splitlines()[-1])
     assert d["config"]["uavs_per_env"] == 32 and d["config"]["envs_total"] == 1048576 and d["config"]["envs_per_gpu"] == 131072
     assert d["scaling"] == "strong"
+
+
+def test_output_sample_keeps_the_same_envs_of_every_array_within_the_budget(monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    import torch
+
+    gen = torch.Generator().manual_seed(0)
+    arrays = dict(obs=torch.rand((1000, 8, 10), generator=gen), reward=torch.rand((1000, 8), generator=gen, dtype=torch.float64),
+                  done=torch.randint(0, 2, (1000, 8), generator=gen, dtype=torch.uint8))
+    whole = bench.output_sample(arrays)
+    assert np.array_equal(whole["env_index"], np.arange(1000)) and whole["done"].dtype == np.float32
+    assert whole["reward"].dtype == np.float64 and np.array_equal(whole["obs"], arrays["obs"].numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100 * (8 + 8 * 10 * 4 + 8 * 8 + 8 * 4))
+    a, b = bench.output_sample(arrays), bench.output_sample(arrays)
+    idx = a["env_index"].astype(np.int64)
+    assert len(idx) == 100 and np.all(np.diff(idx) > 0) and all(np.array_equal(a[k], b[k]) for k in a)
+    for k, v in arrays.items():
+        assert np.array_equal(a[k], v.numpy()[idx])
+
+
+def test_bench_rejects_steps_it_would_not_time():
+    for extra in (["--steps", "0"], ["--workload", "c5r", "--steps", "3"], ["--impl", "reference", "--dump-outputs", "x"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120,
+                             cwd=ROOT)
+        assert out.returncode == 2 and "error" in out.stderr and out.stdout == ""
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("headline", ["rollout", "per_step"])
+def test_dump_outputs_repeat_and_follow_steps(tmp_path, headline):
+    """Two runs with the same arguments write the same arrays; a different --steps writes different ones."""
+
+    def run(steps, name):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1", "--no-cpu-baseline",
+                              "--no-acting", "--headline", headline, "--dump-outputs", str(tmp_path / name)],
+                             capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == steps
+        files = sorted(os.listdir(tmp_path / name))
+        assert files == ["done.npy", "env_index.npy", "obs.npy", "reward.npy"]
+        return {f[:-4]: np.load(tmp_path / name / f) for f in files}
+
+    a, b, c = run(3, "a"), run(3, "b"), run(5, "c")
+    assert a["obs"].shape == (65536, 8, 10) and a["obs"].dtype == np.float32
+    assert sum(v.nbytes for v in a.values()) <= 64e6
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
+    assert not np.array_equal(a["obs"], c["obs"])

@@ -1,6 +1,8 @@
 """CPU: oracle/uav_oracle.c replayed against the golden vectors the literal reference produced
 (oracle/gen_golden.py).  Everything is compared for EXACT equality — flags, float32 positions, float64
 velocities, float64 rewards and float64 observations."""
+import json
+
 import numpy as np
 import pytest
 
@@ -79,70 +81,67 @@ def test_golden_cases_exercise_the_interesting_events():
     assert ev["done"] > 1000 and ev["resets"] > 10 and ev["reach"] > 10 and ev["coll"] > 10 and ev["parked"] > 1000
 
 
-@pytest.mark.skipif(not R.reference_available(), reason="reference checkout only exists in the build container")
-@pytest.mark.parametrize("n", [3, 7])
-def test_oracle_matches_live_reference(n):
-    """Where the reference is present, regenerate a small case live (fresh seed) and compare."""
+def _live_digests():
     from oracle import gen_golden as G
 
-    case = dict(name="live", N=n, E=4, T=120, seed=900 + n, evaluate=0, reset_mode=O.RESET_ON_DONE0, max_steps=60)
-    res = G.run_reference_multi(case)
-    cfg = O.multi_config(4, n, reset_mode=O.RESET_ON_DONE0, max_episode_steps=60, reset_source=O.SOURCE_POOL)
-    orc = O.Oracle(cfg)
-    pool = O.State(G.POOL, n)
-    for f in ("pos", "vel", "tgt", "init", "prev", "flags"):
-        getattr(orc.state, f)[...] = res["init_" + f]
-        getattr(pool, f)[...] = res["pool_" + f]
-    orc.state.episode[...] = 1
-    orc.set_pool(pool)
-    for t in range(case["T"]):
-        out = orc.step(res["action"][t], want_final_obs=True)
-        assert np.array_equal(out["done"], res["done"][t])
-        assert np.array_equal(out["reward"], res["reward"][t])
-        assert np.array_equal(out["obs"], res["obs"][t])
-        assert np.array_equal(out["final_obs"], res["final_obs"][t])
-        assert np.array_equal(orc.state.pos, res["pos"][t])
-        assert np.array_equal(orc.state.vel, res["vel"][t])
+    with open(G.LIVE_DIGESTS) as f:
+        return json.load(f)
 
 
-@pytest.mark.skipif(not R.reference_available(), reason="needs the reference (checkout or oracle/_ref)")
+@pytest.mark.parametrize("n", [3, 7])
+def test_oracle_matches_live_reference(n):
+    """A small pool-reset case on fresh seeds: where the reference is present it runs live and every step is compared
+    exactly; everywhere, every step must reproduce the stored digest of the exact input and output bytes."""
+    from oracle import gen_golden as G
+
+    case = G.live_multi_case(n)
+    res = G.run_reference_multi(case) if R.reference_available() else None
+    want = _live_digests()["live_multi"][str(n)]
+    for t, (a, out, st) in enumerate(G.oracle_live_multi(case)):
+        if res is not None:
+            assert np.array_equal(a, res["action"][t])
+            assert np.array_equal(out["done"], res["done"][t])
+            assert np.array_equal(out["reward"], res["reward"][t])
+            assert np.array_equal(out["obs"], res["obs"][t])
+            assert np.array_equal(out["final_obs"], res["final_obs"][t])
+            assert np.array_equal(st.pos, res["pos"][t])
+            assert np.array_equal(st.vel, res["vel"][t])
+        assert G.live_multi_digest(a, out, st) == want[t], f"step {t} differs from the stored record"
+    assert t + 1 == len(want) == case["T"]
+
+
 @pytest.mark.parametrize("trial", range(6))
 def test_oracle_matches_live_reference_with_random_constructor_arguments(trial):
-    """Non-default worlds against the LITERAL reference, live: box, speed / acceleration bounds, collider radius, sensing
-    range and N drawn at random (crowded enough for collisions, goal reaches and parked UAVs); every output and the
-    whole state compared for exact equality at every step.  (HARD_COLLISION_RADIUS is a module constant of the
-    reference, multi_uav_world_2d.py:8, so it stays 0.5.)"""
-    rng = np.random.default_rng(4100 + trial)
-    n = int(rng.choice([2, 3, 6, 9, 12, 17]))
-    kw = dict(x_size=float(rng.uniform(10, 40)), y_size=float(rng.uniform(10, 40)), max_speed=float(rng.uniform(3, 20)),
-              max_acceleration=float(rng.uniform(1, 12)), collider_radius=float(rng.uniform(0.3, 1.5)),
-              d_sense=float(rng.choice([rng.uniform(1.0, 4.0), rng.uniform(6, 40)])))
-    _, MultiUAVWorld2D = R.load_reference()
-    env = MultiUAVWorld2D(num_agents=n, **kw)
-    env.reset()
-    st = O.sample_multi_states(1, n, rng, x_size=kw["x_size"], y_size=kw["y_size"], collider_radius=kw["collider_radius"],
-                               region=min(kw["x_size"], kw["y_size"]) / 3)
-    R.inject_multi(env, st.pos[0], st.vel[0], st.tgt[0], st.init[0], st.prev[0], st.flags[0])
-    orc = O.Oracle(O.multi_config(1, n, **kw))
-    orc.state = st.copy()
-    assert np.array_equal(orc.observe()[0], np.stack([env._get_obs(a) for a in env.agent_list]))
-    evaluate = bool(trial % 2)
+    """Non-default worlds: box, speed / acceleration bounds, collider radius, sensing range and N drawn at random (crowded
+    enough for collisions, goal reaches and parked UAVs).  Where the reference is present it is stepped live beside the
+    oracle and every output and the whole state are compared for exact equality at every step; everywhere, the drawn
+    world and every step must reproduce the stored digest of the exact bytes.  (HARD_COLLISION_RADIUS is a module
+    constant of the reference, multi_uav_world_2d.py:8, so it stays 0.5.)"""
+    from oracle import gen_golden as G
+
+    want = _live_digests()["random_world"][str(trial)]
+    gen = G.oracle_random_world(trial)
+    setup = next(gen)
+    n, kw, st = setup["n"], setup["kw"], setup["state"]
+    assert (n, kw) == (want["n"], want["kw"]) and G.random_world_setup_digest(setup) == want["setup"]
+    env = None
+    if R.reference_available():
+        _, MultiUAVWorld2D = R.load_reference()
+        env = MultiUAVWorld2D(num_agents=n, **kw)
+        env.reset()
+        R.inject_multi(env, st.pos[0], st.vel[0], st.tgt[0], st.init[0], st.prev[0], st.flags[0])
+        assert np.array_equal(setup["obs0"], np.stack([env._get_obs(a) for a in env.agent_list]))
     events = 0
-    for t in range(250):
-        if t % 3:
-            a = np.clip((orc.state.tgt[0] - orc.state.pos[0]) * 1.2 + rng.normal(0, 0.4, (n, 2)), -kw["max_speed"], kw["max_speed"])
-        else:
-            a = rng.uniform(-kw["max_speed"], kw["max_speed"], (n, 2))
-        f64 = trial >= 3  # half of the trials feed float64 actions that float32 cannot hold (uavo_step_f64act)
-        a = a.astype(np.float64) if f64 else a.astype(np.float32)
-        o, r, d, _ = env.step([a[i].astype(np.float64) for i in range(n)], evaluate=evaluate)
-        out = orc.step_f64(a[None], evaluate=evaluate) if f64 else orc.step(a[None], evaluate=evaluate)
-        assert np.array_equal(out["done"][0], np.array(d, np.uint8)), f"done flags, step {t}"
-        assert np.array_equal(out["reward"][0], np.array(r, np.float64)), f"reward, step {t}"
-        assert np.array_equal(out["obs"][0], np.stack(o)), f"observation, step {t}"
-        pos, vel, tgt, ini, prv, flg = R.extract_multi(env)
-        assert np.array_equal(orc.state.pos[0], pos) and np.array_equal(orc.state.vel[0], vel), f"state, step {t}"
-        assert np.array_equal(orc.state.prev[0], prv) and np.array_equal(orc.state.flags[0], flg), f"latches, step {t}"
-        assert int(orc.state.coll[0]) == env.collision_count and int(orc.state.reach[0]) == env.target_reach_count
-        events += int(np.sum(d)) + int(flg.sum())
-    assert events > 0
+    for t, (a, out, s) in enumerate(gen):
+        if env is not None:
+            o, r, d, _ = env.step([a[i].astype(np.float64) for i in range(n)], evaluate=setup["evaluate"])
+            assert np.array_equal(out["done"][0], np.array(d, np.uint8)), f"done flags, step {t}"
+            assert np.array_equal(out["reward"][0], np.array(r, np.float64)), f"reward, step {t}"
+            assert np.array_equal(out["obs"][0], np.stack(o)), f"observation, step {t}"
+            pos, vel, tgt, ini, prv, flg = R.extract_multi(env)
+            assert np.array_equal(s.pos[0], pos) and np.array_equal(s.vel[0], vel), f"state, step {t}"
+            assert np.array_equal(s.prev[0], prv) and np.array_equal(s.flags[0], flg), f"latches, step {t}"
+            assert int(s.coll[0]) == env.collision_count and int(s.reach[0]) == env.target_reach_count
+        assert G.random_world_digest(a, out, s) == want["steps"][t], f"step {t} differs from the stored record"
+        events += int(out["done"].sum()) + int(s.flags.sum())
+    assert t + 1 == len(want["steps"]) and events > 0
