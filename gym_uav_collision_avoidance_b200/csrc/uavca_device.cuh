@@ -26,7 +26,13 @@ constexpr int kMinBlocksPerSM = UAVCA_MINB;  // step kernel: caps registers per 
 constexpr unsigned kFull = 0xffffffffu;
 constexpr unsigned kMaxResetAttempts = 4096u;  // the reference would loop forever in an over-crowded box
 
-enum : int { kStreamPos = 0, kStreamTgt = 1, kStreamVel = 2, kStreamAct = 3 };
+// Philox4x32-10 streams.  Every key is a seed the caller picks, so the streams are kept apart by their counters alone:
+// each consumer puts its own tag in the upper half of counter word 2 (philox4x32_10 / philox_indexed below).
+//   reset    (env, episode, stream << 16 | uav, attempt)         stream 0..2, uav < 2^16
+//   actions  (env, t >> 1, 3 << 16 | uav, t >> 33)                uav < 2^16
+//   policy   (row, ctr, 4 << 16 | row >> 32, ctr >> 32)          row < 2^48     (uavca_policy.cu)
+//   sampler  (sample, ctr, 5 << 16 | sample >> 32, ctr >> 32)    sample < 2^48  (replay_sample_kernel)
+enum : int { kStreamPos = 0, kStreamTgt = 1, kStreamVel = 2, kStreamAct = 3, kStreamPolicy = 4, kStreamSample = 5 };
 
 // Constants derived once on the host from uavca_config (capi.cu: derive_consts).
 struct Consts {
@@ -317,6 +323,12 @@ __device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_
     k1 += 0xBB67AE85u;
   }
   return make_uint4(c0, c1, c2, c3);
+}
+// The block of stream `tag` (kStreamPolicy, kStreamSample) for a 48-bit index and a 64-bit counter.
+__device__ __forceinline__ uint4 philox_indexed(int tag, unsigned long long index, unsigned long long ctr, uint32_t k0,
+                                                uint32_t k1) {
+  return philox4x32_10((uint32_t)index, (uint32_t)ctr, ((uint32_t)tag << 16) | (uint32_t)(index >> 32), (uint32_t)(ctr >> 32),
+                       k0, k1);
 }
 
 __device__ __forceinline__ double u53(uint32_t a, uint32_t b) {

@@ -775,8 +775,9 @@ __global__ void __launch_bounds__(kPushThreads) replay_push_kernel(const V* obs,
 
 // Replay sampling (ReplayMemory.sample, pytorch_sac_temp/replay_memory.py:21-24; ReplayBuffer.get_batch with its recency
 // weighting, pytorch_ddpg/buffer_tensor.py:65-90): draw `batch` slots and gather the five arrays in ONE launch.  Ring head
-// and fill level are read on the device (ring_meta), the draws come from Philox4x32-10 keyed by (seed, sample, draw +
-// appends so far), so a learner step captured in a CUDA graph samples fresh transitions from the ring as it grows.
+// and fill level are read on the device (ring_meta), the draws come from the sampler's Philox4x32-10 stream keyed by (seed,
+// sample, draw + appends so far) (uavca_device.cuh), so a learner step captured in a CUDA graph samples fresh transitions
+// from the ring as it grows.  An empty ring yields slot 0.
 // 16 threads per sample: they share the slot and copy the rows element-wise.
 constexpr int kSampleLanes = 16;
 __global__ void __launch_bounds__(kThreads) replay_sample_kernel(const float* r_obs, const float* r_act, const float* r_rew,
@@ -790,7 +791,7 @@ __global__ void __launch_bounds__(kThreads) replay_sample_kernel(const float* r_
   if (j >= batch) return;
   const long long head = meta[0], size = meta[2];
   const unsigned long long ctr = draw + (unsigned long long)meta[3];
-  const uint4 r = philox4x32_10((uint32_t)j, (uint32_t)(j >> 32), (uint32_t)ctr, (uint32_t)(ctr >> 32), seed_lo, seed_hi);
+  const uint4 r = philox_indexed(kStreamSample, (unsigned long long)j, ctr, seed_lo, seed_hi);
   long long slot = 0;
   if (size > 0) {
     if (recency) {

@@ -28,9 +28,11 @@
 //   behind it; only the layer-1 epilogue (350 cycles, it needs the A2 buffer layer 2 reads) leaves the tensor pipe idle.
 //
 // W2 (fp16, 128 KB) stays resident in shared memory for the CTA's lifetime.  The tensor-core operands (W1 | b1, W2,
-// activations, W3) are fp16 with fp32 accumulation (11 significand bits, like TF32); b2 and b3 act in fp32: the policy is the learner's side of the
-// boundary, not part of the env-step parity contract; tests compare against the fp32 PyTorch policy at 2e-2
-// absolute on (mean, log_std) — measured 3e-4.
+// activations, W3) are fp16 with fp32 accumulation (11 significand bits, like TF32).  b2 and b3 are fp16 too (rounded on
+// the host like every operand) but are added in fp32, and the second hidden layer reaches the heads unrounded (fp32).  The
+// policy is the learner's side of the boundary, not part of the env-step parity contract: tests/test_acting_kernels_gpu.py
+// holds the heads to a float64 emulation of exactly these rounding points (a per-row bound from the fp32 accumulation,
+// ~1e-4 for O(1) heads) and to the unquantised float64 policy (a bound from the 2^-11 rounding of every fp16 operand).
 #include <cuda_fp16.h>
 
 #include <atomic>
@@ -228,7 +230,7 @@ struct Args {
   float* head;          // [M][4] (mean0, mean1, log_std0, log_std1) or nullptr
   long long M;
   unsigned seed_lo, seed_hi;
-  unsigned long long ctr;               // Philox counter words 2,3 = ctr + *ctr_dev
+  unsigned long long ctr;               // Philox call counter = ctr + *ctr_dev (kStreamPolicy layout, uavca_device.cuh)
   const unsigned long long* ctr_dev;    // nullable
 };
 
@@ -545,8 +547,8 @@ __global__ void __launch_bounds__(kThreads, 1) policy_act_kernel(const __grid_co
         if (a.noise) {
           const float2 z = reinterpret_cast<const float2*>(a.noise)[row];
           e0 = z.x; e1 = z.y;
-        } else {  // Box-Muller on one Philox4x32-10 block keyed by (seed, row, call counter)
-          const uint4 rn = philox4x32_10((uint32_t)row, (uint32_t)(row >> 32), (uint32_t)ctr, (uint32_t)(ctr >> 32), a.seed_lo, a.seed_hi);
+        } else {  // Box-Muller on one block of the policy's Philox4x32-10 stream keyed by (seed, row, call counter)
+          const uint4 rn = philox_indexed(kStreamPolicy, (unsigned long long)row, ctr, a.seed_lo, a.seed_hi);
           const float u1 = ((float)(rn.x >> 8) + 0.5f) * (1.0f / 16777216.0f);
           const float u2 = ((float)(rn.y >> 8) + 0.5f) * (1.0f / 16777216.0f);
           const float rad = sqrtf(-2.0f * __logf(u1));

@@ -65,7 +65,10 @@ class DeviceReplay:
         """`memory.sample(batch_size)` in ONE launch with no host synchronisation (`uavca_replay_sample`): the slots are
         drawn on the device from Philox4x32-10 keyed by (seed, sample, draws so far + appends so far) against the head and
         fill level in `self.meta`, so a learner step captured in a CUDA graph keeps sampling fresh transitions as the ring
-        grows.  Returns (state, action, reward, next_state, mask[, index]); `out` reuses a previous result's tensors."""
+        grows.  Returns (state, action, reward, next_state, mask[, index]); `out` reuses a previous result's tensors.
+        Uniform slot: (x * size) >> 32 of a 32-bit draw x; recency-weighted: age = floor(sqrt((x + 0.5) / 2^32) * size),
+        at most size - 1, counted from the oldest slot (`head` once the ring is full).  An empty ring cannot raise here
+        without a host synchronisation: every slot is 0 and the batch holds ring row 0 (zeros until the first append)."""
         if out is None:
             kw = dict(dtype=torch.float32, device=self.device)
             out = (torch.empty((batch_size, self.obs_dim), **kw), torch.empty((batch_size, self.act_dim), **kw),

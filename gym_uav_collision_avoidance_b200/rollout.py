@@ -82,6 +82,20 @@ class FusedGaussianPolicy:
 
     @torch.no_grad()
     def refresh(self):
+        """Re-pack the weights after the learner updated the policy.  The packed operands are rewritten in place, so an
+        acting step captured in a CUDA graph before the update acts with the new weights when replayed."""
+        packed = self._pack()
+        if not hasattr(self, "w1"):
+            for name, t in packed.items():
+                setattr(self, name, t)
+            return
+        for name, t in packed.items():
+            dst = getattr(self, name)
+            if dst.device != t.device:
+                raise ValueError("the policy moved to another device: build a new FusedGaussianPolicy")
+            dst.copy_(t)
+
+    def _pack(self) -> dict:
         p = self.policy
         if hasattr(p, "l1") and hasattr(p, "l3"):
             # deterministic TD3-style actor (pytorch_td3_temp/td3.py:14-27: l1, l2, l3, tanh): the same kernel with the
@@ -98,27 +112,39 @@ class FusedGaussianPolicy:
             raise ValueError("the policy must live on a CUDA device")
         dev, h = w1.device, torch.float16
         # fp16 K-major operands; every bias rides in an extra input column (include/uavca.h)
-        self.w1 = torch.zeros((256, 16), dtype=h, device=dev)
-        self.w1[:, :10] = w1.to(h)
-        self.w1[:, 10] = lin1.bias.to(h)
-        self.w2 = w2.to(h).contiguous()
-        self.w2b = torch.zeros((256, 16), dtype=h, device=dev)
-        self.w2b[:, 0] = lin2.bias.to(h)
-        self.w3 = torch.zeros((16, 256), dtype=h, device=dev)
-        self.w3[0:2] = mean_w.to(h)
-        self.w3[2:4] = std_w.to(h)
-        self.w3b = torch.zeros((16, 16), dtype=h, device=dev)
-        self.w3b[0:2, 0] = mean_b.to(h)
-        self.w3b[2:4, 0] = std_b.to(h)
+        w1p = torch.zeros((256, 16), dtype=h, device=dev)
+        w1p[:, :10] = w1.to(h)
+        w1p[:, 10] = lin1.bias.to(h)
+        w2b = torch.zeros((256, 16), dtype=h, device=dev)
+        w2b[:, 0] = lin2.bias.to(h)
+        w3 = torch.zeros((16, 256), dtype=h, device=dev)
+        w3[0:2] = mean_w.to(h)
+        w3[2:4] = std_w.to(h)
+        w3b = torch.zeros((16, 16), dtype=h, device=dev)
+        w3b[0:2, 0] = mean_b.to(h)
+        w3b[2:4, 0] = std_b.to(h)
+        return dict(w1=w1p, w2=w2.to(h).contiguous(), w2b=w2b, w3=w3, w3b=w3b)
 
     def act(self, state: torch.Tensor, evaluate: bool = False, out: Optional[torch.Tensor] = None,
             noise: Optional[torch.Tensor] = None, head: Optional[torch.Tensor] = None) -> torch.Tensor:
         """state [M, 10] float32 CUDA -> action [M, 2] in (-1, 1).  `noise` [M, 2] overrides the Philox draws (tests);
-        `head` [M, 4] receives (mean, log_std)."""
+        `head` [M, 4] receives (mean, log_std).  Every tensor must be float32 on the policy's device; anything else
+        raises ValueError before the kernel is launched (the kernel reads and writes raw float32 rows)."""
         from . import ops
 
+        dev = self.w2.device
+        if state.dtype != torch.float32 or state.device != dev:
+            raise ValueError(f"state must be float32 on {dev}, got {state.dtype} on {state.device}")
+        if state.numel() % 10:
+            raise ValueError(f"state holds {state.numel()} values, not a whole number of 10-feature observations")
         state = state.contiguous()
         M = state.numel() // 10
+        for name, t, width in (("out", out, 2), ("noise", noise, 2), ("head", head, 4)):
+            if t is None:
+                continue
+            if t.dtype != torch.float32 or t.device != dev or tuple(t.shape) != (M, width) or not t.is_contiguous():
+                raise ValueError(f"{name} must be a contiguous float32 [{M}, {width}] tensor on {dev}, "
+                                 f"got {t.dtype} {tuple(t.shape)} on {t.device}")
         if out is None:
             out = torch.empty((M, 2), dtype=torch.float32, device=state.device)
         ops.policy_act(state, self.w1, self.w2, self.w2b, self.w3, self.w3b, noise, self.seed, self.calls, self.counter,

@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define UAVCA_VERSION 202
+#define UAVCA_VERSION 203
 
 /* world kinds */
 #define UAVCA_KIND_MULTI 0  /* MultiUAVWorld2D: N UAVs per env, 10-feature observation */
@@ -232,9 +232,12 @@ int uavca_replay_push_dev(const float* obs, const float* action, const float* re
 
 /* Draw `batch` transitions from the ring and gather the five arrays in ONE launch ("next" row; replaces ReplayMemory.sample,
  * pytorch_sac_temp/replay_memory.py:21-24, and ReplayBuffer.get_batch, pytorch_ddpg/buffer_tensor.py:65-90).  Head and fill
- * level are read from ring_meta on the device; the slots come from Philox4x32-10 keyed by (seed, sample index, draw +
- * appends so far), uniformly over the filled slots (with replacement) or, with recency_weighted != 0, with probability
- * rising linearly with recency (the `unbalance_p` scheme of buffer_tensor.py:78-87).  No host synchronisation: safe inside a
+ * level are read from ring_meta on the device; the slots come from word 0 (x) of the Philox4x32-10 block with key seed and
+ * counter (j, ctr, 5 << 16 | j >> 32, ctr >> 32) for sample j and ctr = draw + appends so far (ring_meta[3]), uniformly over
+ * the filled slots with replacement ((x * size) >> 32) or, with recency_weighted != 0, with probability rising linearly
+ * with recency (the `unbalance_p` scheme of buffer_tensor.py:78-87: age = floor(sqrt((x + 0.5) / 2^32) * size), at most
+ * size - 1, counted from the oldest slot).  The tag 5 in counter word 2 keeps the stream apart from every other Philox
+ * stream of the library (env resets 0..2, rollout actions 3, policy noise 4) whatever the seeds.  No host synchronisation: safe inside a
  * CUDA graph of a learner step.  out_*: float [batch][obs_dim] / [batch][act_dim] / [batch]; out_index (nullable) int64
  * [batch] receives the slots.  An empty ring yields slot 0. */
 int uavca_replay_sample(const float* ring_obs, const float* ring_action, const float* ring_reward, const float* ring_next_obs,
@@ -266,9 +269,10 @@ int uavca_step_multi_replay(uavca_handle* h, void* state, const float* action, i
  *   w2  fp16 [256][256] : linear2.weight;            w2b fp16 [256][16] : linear2.bias in column 0, zeros;
  *   w3  fp16 [16][256]  : rows 0,1 mean_linear.weight, rows 2,3 log_std_linear.weight, zeros;
  *   w3b fp16 [16][16]   : mean_linear.bias, log_std_linear.bias in column 0 of rows 0..3, zeros;
- *   noise float [M][2] standard-normal draws or NULL (then Philox4x32-10 keyed by seed, row and
- *   counter + *counter_dev; counter_dev is a nullable DEVICE uint64 the caller advances between calls, which keeps
- *   a CUDA-graph replay of the call from repeating its noise);
+ *   noise float [M][2] standard-normal draws or NULL: then Box-Muller on the Philox4x32-10 block with key seed and
+ *   counter (row, ctr, 4 << 16 | row >> 32, ctr >> 32), ctr = counter + *counter_dev (tag 4: no other Philox stream of
+ *   the library can produce that counter); counter_dev is a nullable DEVICE uint64 the caller advances between calls,
+ *   which keeps a CUDA-graph replay of the call from repeating its noise;
  *   action float [M][2] = tanh(mean + exp(clamp(log_std, -20, 2)) * noise);  head (nullable) float [M][4] = mean, log_std.
  * No handle: weights and buffers belong to the caller. */
 int uavca_policy_act(const float* obs, int64_t M, const void* w1, const void* w2, const void* w2b, const void* w3,
