@@ -209,22 +209,23 @@ __device__ __forceinline__ float fast_atan2(float y, float x) {
 }
 
 // Two atan2 at once: the polynomial runs on Blackwell's packed FP32 pipe (FMUL2/FFMA2, two lanes per instruction);
-// octant reduction and fix-up stay scalar.  Same arithmetic per element as fast_atan2.
-__constant__ float2 kAtanC[9] = {
-    {0.0029206890612840652f, 0.0029206890612840652f}, {-0.016367916017770767f, -0.016367916017770767f},
-    {0.04321184381842613f, 0.04321184381842613f},     {-0.07552213221788406f, -0.07552213221788406f},
-    {0.10666003823280334f, 0.10666003823280334f},     {-0.14211055636405945f, -0.14211055636405945f},
-    {0.19993773102760315f, 0.19993773102760315f},     {-0.33333152532577515f, -0.33333152532577515f},
-    {1.0f, 1.0f}};
-
+// octant reduction and fix-up stay scalar.  Same arithmetic per element as fast_atan2.  The coefficients are literals:
+// FFMA2 takes a 32-bit immediate for both lanes, where a __constant__ table costs an LDC per coefficient and call.
 __device__ __forceinline__ float2 fast_atan2_pair(float y0, float x0, float y1, float x1) {
   const float ax0 = fabsf(x0), ay0 = fabsf(y0), ax1 = fabsf(x1), ay1 = fabsf(y1);
   const float mx0 = fmaxf(ax0, ay0), mn0 = fminf(ax0, ay0), mx1 = fmaxf(ax1, ay1), mn1 = fminf(ax1, ay1);
   const float2 t = make_float2(__fdividef(mn0, mx0 + 1e-37f), __fdividef(mn1, mx1 + 1e-37f));
   const float2 s = __fmul2_rn(t, t);
-  float2 p = kAtanC[0];
-#pragma unroll
-  for (int k = 1; k < 9; ++k) p = __ffma2_rn(p, s, kAtanC[k]);
+  auto both = [](float v) { return make_float2(v, v); };
+  float2 p = both(0.0029206890612840652f);
+  p = __ffma2_rn(p, s, both(-0.016367916017770767f));
+  p = __ffma2_rn(p, s, both(0.04321184381842613f));
+  p = __ffma2_rn(p, s, both(-0.07552213221788406f));
+  p = __ffma2_rn(p, s, both(0.10666003823280334f));
+  p = __ffma2_rn(p, s, both(-0.14211055636405945f));
+  p = __ffma2_rn(p, s, both(0.19993773102760315f));
+  p = __ffma2_rn(p, s, both(-0.33333152532577515f));
+  p = __ffma2_rn(p, s, both(1.0f));
   float2 r = __fmul2_rn(t, p);
   r.x = (ay0 > ax0) ? (1.57079637050628662f - r.x) : r.x;
   r.y = (ay1 > ax1) ? (1.57079637050628662f - r.y) : r.y;

@@ -250,7 +250,14 @@ __global__ void __launch_bounds__(kThreads, kMinBlocksPerSM) step_multi_ring_ker
 // of K-1 dependent launches and 66 of the 107 algorithmic bytes per UAV-step (the state round trip and, with Philox
 // actions, the action read).  Runs the very same step_core as the one-step kernel, so the results are bit-identical
 // to K single steps.
+//
+// PLAIN: the launch of an open-loop driver loop (bench.py, run_multi.py): cartesian actions (block actions as given,
+// Philox actions scaled to the action box before step_core sees them), no final_obs, reset_mask, action_out or score
+// tracking.  Those options then cost nothing per step; every other combination runs the general instance, which tests
+// them at run time.
+template <bool PLAIN>
 struct RolloutIO {
+  static constexpr bool kPlain = PLAIN;
   const KernelArgs& a;
   const RolloutArgs& r;
   const Lane& L;
@@ -258,24 +265,26 @@ struct RolloutIO {
   Uav cur;
   float2 act;
   int steps;
-  int k;  // step of the launch: outputs go to slot k of the [K][...] blocks (one 64-bit multiply-add per store; running
-          // pointers were tried and cost ten more live registers across step_core: 300 bytes of spills at 64 registers)
+  int k;          // step of the launch: outputs go to slot k of the [K][...] blocks
+  long long km;   // k * M, warp-uniform: the slot bases are uniform-datapath arithmetic, only the lane's offset is added
+                  // per lane (running per-lane pointers were tried and cost ten more live registers across step_core: 300
+                  // bytes of spills at 64 registers)
   __device__ __forceinline__ Uav load_uav() const { return cur; }
   __device__ __forceinline__ float2 load_action() const { return act; }
   __device__ __forceinline__ int load_steps() const { return steps; }
   __device__ __forceinline__ void loads_done() const {}
   __device__ __forceinline__ void store_reward_done(float rw, bool done) const {
     if (L.valid) {
-      st_stream(a.io.reward + (size_t)k * r.M + L.m, rw);
-      st_stream(a.io.done + (size_t)k * r.M + L.m, (uint8_t)done);
+      st_stream((a.io.reward + km) + (unsigned)L.m, rw);
+      st_stream((a.io.done + km) + (unsigned)L.m, (uint8_t)done);
     }
   }
-  __device__ __forceinline__ bool wants_final() const { return a.io.final_obs != nullptr; }
+  __device__ __forceinline__ bool wants_final() const { return !PLAIN && a.io.final_obs != nullptr; }
   __device__ __forceinline__ void put_own(float2 o01, float2 o23) const { stage_own(stage, L.lane, o01, o23); }
   __device__ __forceinline__ void put_neighbours(const ObsTail& n) const { stage_neighbours(stage, L.lane, n); }
   __device__ __forceinline__ void commit(float* g) const {
     __syncwarp();
-    flush_rows(stage, g + (size_t)k * r.M * UAVCA_OBS_DIM_MULTI, L);
+    flush_warp_rows(stage, (g + km * UAVCA_OBS_DIM_MULTI) + (unsigned)L.warp_m0 * (size_t)UAVCA_OBS_DIM_MULTI, L);
     __syncwarp();
   }
   __device__ __forceinline__ void commit_obs() const { commit(a.io.obs); }
@@ -284,34 +293,58 @@ struct RolloutIO {
   __device__ __forceinline__ void store_target(const Uav&) const {}  // store_state carried the new target already
   __device__ __forceinline__ void store_steps(int v, bool) { steps = v; }
   __device__ __forceinline__ void store_reset(bool rs) const {
-    if (a.io.reset_mask) a.io.reset_mask[(size_t)k * r.B + L.env] = (uint8_t)rs;
+    if (!PLAIN && a.io.reset_mask) a.io.reset_mask[(size_t)k * r.B + L.env] = (uint8_t)rs;
   }
 };
 
-template <int NT, bool FULL>
+// the action slots by their shared-memory address: one 32-bit register per lane, no generic-address conversion per step
+__device__ __forceinline__ void cp_async8(unsigned smem_dst, const void* gsrc) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_dst), "l"(gsrc) : "memory");
+}
+__device__ __forceinline__ float2 lds_float2(unsigned smem_src) {
+  float2 v;
+  asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(smem_src) : "memory");
+  return v;
+}
+
+// Instances of the rollout kernel: the plain launch (RolloutIO) with an action block and with Philox actions, each
+// with its action source fixed at compile time, and one general instance that tests the action source and every option
+// at run time.
+enum RolloutKind : int { kRolloutGeneral = 0, kRolloutPlainBlock = 1, kRolloutPlainPhilox = 2 };
+
+// Everything that does not change from step to step (the lane geometry, the lane's action slot, the warp's row offset)
+// is computed once, before the K loop.
+template <int NT, bool FULL, int KIND>
 __device__ __forceinline__ void rollout_multi_body(const KernelArgs& a, const RolloutArgs& r, const WarpScratch& ws,
-                                                   float* act_smem, int warp_global) {
+                                                   float2* act_smem, int warp_global) {
+  constexpr bool kPlain = KIND != kRolloutGeneral;
+  const bool block = KIND == kRolloutGeneral ? r.action_block != nullptr : KIND == kRolloutPlainBlock;  // warp-uniform
   const Lane L = make_lane<NT, FULL>(a.B, a.N, warp_global);
-  RolloutIO io{a, r, L, ws.stage, load_uav(a.s, L), make_float2(0.f, 0.f), L.valid ? a.s.steps[L.env] : 0, 0};
+  RolloutIO<kPlain> io{a, r, L, ws.stage, load_uav(a.s, L), make_float2(0.f, 0.f), L.valid ? a.s.steps[L.env] : 0, 0, 0};
   cudaTriggerProgrammaticLaunchCompletion();
-  const long long env_global = a.c.env_base + L.env;
+  // Action block: the action of step k+1 travels while step k is computed — by cp.async into a per-lane shared-memory
+  // slot (two slots, alternating), not into registers: at 64 registers ptxas sinks a register prefetch down to its use,
+  // and ncu showed 15 % of the warp-time waiting on that load (profiles/r2_full_rollout_n32.md)
+  const unsigned slot = (unsigned)__cvta_generic_to_shared(act_smem + L.lane);
+  if (block && L.valid) cp_async8(slot, r.action_block + L.m);
+  const long long env_global = a.c.env_base + L.env;  // Philox actions
   uint4 words = make_uint4(0u, 0u, 0u, 0u);
-  // Action block: the action of step k+1 travels while step k is computed — by cp.async into a per-lane shared-memory slot
-  // (two slots, alternating), not into registers: at 64 registers ptxas sinks a register prefetch down to its use, and
-  // ncu showed 15 % of the warp-time waiting on that load (profiles/r2_full_rollout_n32.md).
-  float2* act_slot = reinterpret_cast<float2*>(act_smem) + L.lane;
-  if (r.action_block != nullptr && L.valid) cp_async(act_slot, r.action_block + L.m, 8);
   for (int k = 0; k < r.K; ++k) {
     io.k = k;
-    if (r.action_block != nullptr) {
+    io.km = (long long)k * r.M;
+    if (block) {
       cp_async_wait_all();
-      io.act = L.valid ? act_slot[(k & 1) * 32] : make_float2(0.f, 0.f);
-      if (k + 1 < r.K && L.valid) cp_async(act_slot + ((k + 1) & 1) * 32, r.action_block + (size_t)(k + 1) * r.M + L.m, 8);
+      io.act = L.valid ? lds_float2(slot + (k & 1) * 256) : make_float2(0.f, 0.f);
+      if (k + 1 < r.K && L.valid) cp_async8(slot + ((k + 1) & 1) * 256, (r.action_block + (io.km + r.M)) + (unsigned)L.m);
     } else {
       const unsigned long long t = r.step0 + (unsigned long long)k;
       if (k == 0 || (t & 1ull) == 0ull) words = action_words(r.seed_lo, r.seed_hi, env_global, L.i, t);
       io.act = action_from_words(words, t);
-      if (r.action_out != nullptr && L.valid) st_stream(r.action_out + (size_t)k * r.M + L.m, io.act);
+      if (kPlain) {
+        io.act = map_action(io.act, UAVCA_ACTION_SCALED, a.c);  // what step_core would do with the launch's mode
+      } else if (r.action_out != nullptr && L.valid) {
+        st_stream((r.action_out + io.km) + L.m, io.act);
+      }
     }
     step_core<NT>(a, ws, L, io);
   }
@@ -324,19 +357,19 @@ __device__ __forceinline__ void rollout_multi_body(const KernelArgs& a, const Ro
 #ifndef UAVCA_ROLLOUT_MINB
 #define UAVCA_ROLLOUT_MINB 8
 #endif
-template <int NT>
+template <int NT, int KIND>
 __global__ void __launch_bounds__(kThreads, UAVCA_ROLLOUT_MINB) rollout_multi_kernel(const __grid_constant__ KernelArgs a,
                                                                                   const __grid_constant__ RolloutArgs r) {
   __shared__ __align__(16) float smem[kWarpsPerBlock * kScratchFloats];
-  __shared__ __align__(16) float act_smem[kWarpsPerBlock * 128];  // per warp: two slots of 32 float2 actions
+  __shared__ __align__(16) float2 act_smem[kWarpsPerBlock * 64];  // per warp: two slots of 32 float2 actions
   const WarpScratch ws = warp_scratch(smem);
   const int warp_global = blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
   const int N = NT > 0 ? NT : a.N;
   const bool full = uavs_left(a.B, N, warp_global) >= (32 / N) * N;  // warp-uniform
   cudaGridDependencySynchronize();
-  float* const my_act = act_smem + (threadIdx.x >> 5) * 128;
-  if (full) rollout_multi_body<NT, true>(a, r, ws, my_act, warp_global);
-  else rollout_multi_body<NT, false>(a, r, ws, my_act, warp_global);
+  float2* const my_act = act_smem + (threadIdx.x >> 5) * 64;
+  if (full) rollout_multi_body<NT, true, KIND>(a, r, ws, my_act, warp_global);
+  else rollout_multi_body<NT, false, KIND>(a, r, ws, my_act, warp_global);
 }
 
 // The action stream of uavca_rollout on its own, one step: out[m] = the policy-space action of global step t.
@@ -1129,7 +1162,19 @@ cudaError_t launch_rollout_multi(const KernelArgs& a, const RolloutArgs& r, cuda
     return e != cudaSuccess ? e : cudaGetLastError();
   }
   const int grid = multi_grid(a.B, a.N);
-  UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT>, grid, st, a, r)));
+  const bool block = r.action_block != nullptr;
+  // the plain instance (RolloutIO): the action mode the plain call implies — cartesian block actions, Philox actions
+  // scaled to the action box — and none of the optional outputs or accumulators
+  const bool plain = a.io.final_obs == nullptr && a.io.reset_mask == nullptr && !a.c.track_scores &&
+                     (block ? a.io.action_mode == UAVCA_ACTION_CARTESIAN
+                            : a.io.action_mode == UAVCA_ACTION_SCALED && r.action_out == nullptr);
+  if (block && plain) {
+    UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT, kRolloutPlainBlock>, grid, st, a, r)));
+  } else if (plain) {
+    UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT, kRolloutPlainPhilox>, grid, st, a, r)));
+  } else {
+    UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT, kRolloutGeneral>, grid, st, a, r)));
+  }
   return e != cudaSuccess ? e : cudaGetLastError();
 }
 

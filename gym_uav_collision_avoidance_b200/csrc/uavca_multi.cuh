@@ -651,11 +651,18 @@ template <class IO, class = void>
 struct io_action64 { static constexpr bool value = false; };
 template <class IO>
 struct io_action64<IO, decltype((void)IO::kAction64)> { static constexpr bool value = IO::kAction64; };
+// An I/O policy that declares `static constexpr bool kPlain = true` hands the step cartesian actions (already mapped)
+// and is used only where the launch tracks no scores (Consts::track_scores == 0): neither is then tested at run time.
+template <class IO, class = void>
+struct io_plain { static constexpr bool value = false; };
+template <class IO>
+struct io_plain<IO, decltype((void)IO::kPlain)> { static constexpr bool value = IO::kPlain; };
 
 template <int NT, class IO>
 __device__ __forceinline__ void step_core(const KernelArgs& a, const WarpScratch& ws, const Lane& L, IO& io) {
   const Consts& c = a.c;
   constexpr bool kF64 = io_action64<IO>::value;
+  constexpr bool kPlain = io_plain<IO>::value;
 
   Uav u = io.load_uav();
   float2 act = make_float2(0.f, 0.f);
@@ -664,7 +671,7 @@ __device__ __forceinline__ void step_core(const KernelArgs& a, const WarpScratch
   else act = io.load_action();
   const int steps_new = io.load_steps() + 1;  // multi_uav_world_2d.py:238
   io.loads_done();
-  if constexpr (!kF64) {
+  if constexpr (!kF64 && !kPlain) {
     if (a.io.action_mode != UAVCA_ACTION_CARTESIAN) act = map_action(act, a.io.action_mode, c);
   }
 
@@ -741,7 +748,7 @@ __device__ __forceinline__ void step_core(const KernelArgs& a, const WarpScratch
   if (leader) io.store_reset(rs);
   // per-episode scores the training loops keep on the host (test_sac_multi.py:105: score += rewards[0];
   // :152-156: total_score += rewards[i] * (1 - dones[i])), accumulated per env when asked for
-  if (c.track_scores) {
+  if (!kPlain && c.track_scores) {
     const float live = env_sum((done | !L.valid) ? 0.0f : r, L);
     if (leader) {
       double2 sc = a.s.score[L.env];
