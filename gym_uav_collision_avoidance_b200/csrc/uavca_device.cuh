@@ -118,6 +118,7 @@ struct RolloutArgs {
   unsigned long long step0;    // global index of step k = 0 (Philox counter word; the caller advances it by K)
   long long M;                 // B * N of this launch (stride of one step in the blocks)
   int B;
+  unsigned KM;                 // K * M: end of the plain instances' 32-bit step offsets (set by launch_rollout_multi)
 };
 
 // Device replay ring fed straight from the step kernel (uavca_step_multi_replay): the step that produced a transition

@@ -251,13 +251,9 @@ __global__ void __launch_bounds__(kThreads, kMinBlocksPerSM) step_multi_ring_ker
 // actions, the action read).  Runs the very same step_core as the one-step kernel, so the results are bit-identical
 // to K single steps.
 //
-// PLAIN: the launch of an open-loop driver loop (bench.py, run_multi.py): cartesian actions (block actions as given,
-// Philox actions scaled to the action box before step_core sees them), no final_obs, reset_mask, action_out or score
-// tracking.  Those options then cost nothing per step; every other combination runs the general instance, which tests
-// them at run time.
-template <bool PLAIN>
+// The general instance tests the action source and every option of uavca_rollout (final_obs, reset_mask, action_out,
+// score tracking, any action mode) at run time.
 struct RolloutIO {
-  static constexpr bool kPlain = PLAIN;
   const KernelArgs& a;
   const RolloutArgs& r;
   const Lane& L;
@@ -266,9 +262,7 @@ struct RolloutIO {
   float2 act;
   int steps;
   int k;          // step of the launch: outputs go to slot k of the [K][...] blocks
-  long long km;   // k * M, warp-uniform: the slot bases are uniform-datapath arithmetic, only the lane's offset is added
-                  // per lane (running per-lane pointers were tried and cost ten more live registers across step_core: 300
-                  // bytes of spills at 64 registers)
+  long long km;   // k * M
   __device__ __forceinline__ Uav load_uav() const { return cur; }
   __device__ __forceinline__ float2 load_action() const { return act; }
   __device__ __forceinline__ int load_steps() const { return steps; }
@@ -279,7 +273,7 @@ struct RolloutIO {
       st_stream((a.io.done + km) + (unsigned)L.m, (uint8_t)done);
     }
   }
-  __device__ __forceinline__ bool wants_final() const { return !PLAIN && a.io.final_obs != nullptr; }
+  __device__ __forceinline__ bool wants_final() const { return a.io.final_obs != nullptr; }
   __device__ __forceinline__ void put_own(float2 o01, float2 o23) const { stage_own(stage, L.lane, o01, o23); }
   __device__ __forceinline__ void put_neighbours(const ObsTail& n) const { stage_neighbours(stage, L.lane, n); }
   __device__ __forceinline__ void commit(float* g) const {
@@ -293,63 +287,127 @@ struct RolloutIO {
   __device__ __forceinline__ void store_target(const Uav&) const {}  // store_state carried the new target already
   __device__ __forceinline__ void store_steps(int v, bool) { steps = v; }
   __device__ __forceinline__ void store_reset(bool rs) const {
-    if (!PLAIN && a.io.reset_mask) a.io.reset_mask[(size_t)k * r.B + L.env] = (uint8_t)rs;
+    if (a.io.reset_mask) a.io.reset_mask[(size_t)k * r.B + L.env] = (uint8_t)rs;
   }
+};
+
+// PLAIN: the launch of an open-loop driver loop (bench.py, run_multi.py): cartesian actions (block actions as given,
+// Philox actions scaled to the action box before step_core sees them), no final_obs, reset_mask, action_out or score
+// tracking.  Those options then cost nothing per step.
+// Every per-step address is the lane's element offset off = k * M + m, one 32-bit register advanced by M per step: an
+// address is the parameter base plus off * sizeof (a LEA pair), with no step counter and no 64-bit index arithmetic in
+// the loop.  The launcher runs this instance only where K * M * 10 < 2^31, so the observation offset off * 10 fits too.
+// The observation stage is written and read through its shared-memory address, computed once before the loop.
+struct PlainRolloutIO {
+  static constexpr bool kPlain = true;
+  const KernelArgs& a;
+  const Lane& L;
+  unsigned stage;  // shared-memory address of the warp's observation stage
+  Uav cur;
+  float2 act;
+  int steps;
+  unsigned off;  // k * M + m
+  __device__ __forceinline__ Uav load_uav() const { return cur; }
+  __device__ __forceinline__ float2 load_action() const { return act; }
+  __device__ __forceinline__ int load_steps() const { return steps; }
+  __device__ __forceinline__ void loads_done() const {}
+  __device__ __forceinline__ void store_reward_done(float rw, bool done) const {
+    if (L.valid) {
+      st_stream(a.io.reward + off, rw);
+      st_stream(a.io.done + off, (uint8_t)done);
+    }
+  }
+  __device__ __forceinline__ bool wants_final() const { return false; }
+  __device__ __forceinline__ void put_own(float2 o01, float2 o23) const { stage_own(stage, L.lane, o01, o23); }
+  __device__ __forceinline__ void put_neighbours(const ObsTail& n) const { stage_neighbours(stage, L.lane, n); }
+  __device__ __forceinline__ void commit_obs() const {
+    __syncwarp();
+    flush_warp_rows(stage, a.io.obs + (off - (unsigned)L.lane) * (unsigned)UAVCA_OBS_DIM_MULTI, L);  // (k * M + warp_m0) * 10
+    __syncwarp();
+  }
+  __device__ __forceinline__ void commit_final() const {}
+  __device__ __forceinline__ void store_state(const Uav& u) { cur = u; }
+  __device__ __forceinline__ void store_target(const Uav&) const {}  // store_state carried the new target already
+  __device__ __forceinline__ void store_steps(int v, bool) { steps = v; }
+  __device__ __forceinline__ void store_reset(bool) const {}
 };
 
 // the action slots by their shared-memory address: one 32-bit register per lane, no generic-address conversion per step
 __device__ __forceinline__ void cp_async8(unsigned smem_dst, const void* gsrc) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_dst), "l"(gsrc) : "memory");
 }
-__device__ __forceinline__ float2 lds_float2(unsigned smem_src) {
-  float2 v;
-  asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(smem_src) : "memory");
-  return v;
-}
 
-// Instances of the rollout kernel: the plain launch (RolloutIO) with an action block and with Philox actions, each
-// with its action source fixed at compile time, and one general instance that tests the action source and every option
-// at run time.
+// Instances of the rollout kernel: the plain launch (PlainRolloutIO) with an action block and with Philox actions, each
+// with its action source fixed at compile time, and one general instance (RolloutIO) that tests the action source and
+// every option at run time.
 enum RolloutKind : int { kRolloutGeneral = 0, kRolloutPlainBlock = 1, kRolloutPlainPhilox = 2 };
 
 // Everything that does not change from step to step (the lane geometry, the lane's action slot, the warp's row offset)
 // is computed once, before the K loop.
+// Action block: the action of step k+1 travels while step k is computed — by cp.async into a per-lane shared-memory
+// slot (two slots, alternating), not into registers: at 64 registers ptxas sinks a register prefetch down to its use,
+// and ncu showed 15 % of the warp-time waiting on that load (profiles/r2_full_rollout_n32.md).  The two slots of a lane
+// lie 256 bytes apart in the warp's 512-byte aligned block: the other slot is slot ^ 256.
 template <int NT, bool FULL, int KIND>
 __device__ __forceinline__ void rollout_multi_body(const KernelArgs& a, const RolloutArgs& r, const WarpScratch& ws,
                                                    float2* act_smem, int warp_global) {
-  constexpr bool kPlain = KIND != kRolloutGeneral;
-  const bool block = KIND == kRolloutGeneral ? r.action_block != nullptr : KIND == kRolloutPlainBlock;  // warp-uniform
   const Lane L = make_lane<NT, FULL>(a.B, a.N, warp_global);
-  RolloutIO<kPlain> io{a, r, L, ws.stage, load_uav(a.s, L), make_float2(0.f, 0.f), L.valid ? a.s.steps[L.env] : 0, 0, 0};
-  cudaTriggerProgrammaticLaunchCompletion();
-  // Action block: the action of step k+1 travels while step k is computed — by cp.async into a per-lane shared-memory
-  // slot (two slots, alternating), not into registers: at 64 registers ptxas sinks a register prefetch down to its use,
-  // and ncu showed 15 % of the warp-time waiting on that load (profiles/r2_full_rollout_n32.md)
-  const unsigned slot = (unsigned)__cvta_generic_to_shared(act_smem + L.lane);
-  if (block && L.valid) cp_async8(slot, r.action_block + L.m);
+  unsigned slot = (unsigned)__cvta_generic_to_shared(act_smem + L.lane);
   const long long env_global = a.c.env_base + L.env;  // Philox actions
-  uint4 words = make_uint4(0u, 0u, 0u, 0u);
-  for (int k = 0; k < r.K; ++k) {
-    io.k = k;
-    io.km = (long long)k * r.M;
-    if (block) {
-      cp_async_wait_all();
-      io.act = L.valid ? lds_float2(slot + (k & 1) * 256) : make_float2(0.f, 0.f);
-      if (k + 1 < r.K && L.valid) cp_async8(slot + ((k + 1) & 1) * 256, (r.action_block + (io.km + r.M)) + (unsigned)L.m);
+  if constexpr (KIND != kRolloutGeneral) {
+    PlainRolloutIO io{a, L, (unsigned)__cvta_generic_to_shared(ws.stage), load_uav(a.s, L), make_float2(0.f, 0.f),
+                      L.valid ? a.s.steps[L.env] : 0, (unsigned)L.m};
+    cudaTriggerProgrammaticLaunchCompletion();
+    const unsigned M = (unsigned)r.M;
+    if constexpr (KIND == kRolloutPlainBlock) {
+      const unsigned end = r.KM + (unsigned)L.m;  // end - off is the same in every lane: the loop is warp-uniform
+      if (L.valid) cp_async8(slot, r.action_block + io.off);
+      do {
+        cp_async_wait_all();
+        io.act = L.valid ? lds_float2(slot) : make_float2(0.f, 0.f);
+        const unsigned next = io.off + M;
+        if (next < end && L.valid) cp_async8(slot ^ 256u, r.action_block + next);
+        step_core<NT>(a, ws, L, io);
+        io.off = next;
+        slot ^= 256u;
+      } while (io.off < end);
     } else {
-      const unsigned long long t = r.step0 + (unsigned long long)k;
-      if (k == 0 || (t & 1ull) == 0ull) words = action_words(r.seed_lo, r.seed_hi, env_global, L.i, t);
-      io.act = action_from_words(words, t);
-      if (kPlain) {
-        io.act = map_action(io.act, UAVCA_ACTION_SCALED, a.c);  // what step_core would do with the launch's mode
-      } else if (r.action_out != nullptr && L.valid) {
-        st_stream((r.action_out + io.km) + L.m, io.act);
+      // the Philox counter needs the step index itself: k stays, the addresses still come from the offset alone
+      uint4 words = make_uint4(0u, 0u, 0u, 0u);
+      for (int k = 0; k < r.K; ++k) {
+        const unsigned long long t = r.step0 + (unsigned long long)k;
+        if (k == 0 || (t & 1ull) == 0ull) words = action_words(r.seed_lo, r.seed_hi, env_global, L.i, t);
+        io.act = map_action(action_from_words(words, t), UAVCA_ACTION_SCALED, a.c);  // what step_core would do with the launch's mode
+        step_core<NT>(a, ws, L, io);
+        io.off += M;
       }
     }
-    step_core<NT>(a, ws, L, io);
+    store_uav(a.s, L, io.cur, true);
+    if (L.valid & (L.i == 0)) a.s.steps[L.env] = io.steps;
+  } else {
+    const bool block = r.action_block != nullptr;  // warp-uniform
+    RolloutIO io{a, r, L, ws.stage, load_uav(a.s, L), make_float2(0.f, 0.f), L.valid ? a.s.steps[L.env] : 0, 0, 0};
+    cudaTriggerProgrammaticLaunchCompletion();
+    if (block && L.valid) cp_async8(slot, r.action_block + L.m);
+    uint4 words = make_uint4(0u, 0u, 0u, 0u);
+    for (int k = 0; k < r.K; ++k) {
+      io.k = k;
+      io.km = (long long)k * r.M;
+      if (block) {
+        cp_async_wait_all();
+        io.act = L.valid ? lds_float2(slot + (k & 1) * 256) : make_float2(0.f, 0.f);
+        if (k + 1 < r.K && L.valid) cp_async8(slot + ((k + 1) & 1) * 256, (r.action_block + (io.km + r.M)) + (unsigned)L.m);
+      } else {
+        const unsigned long long t = r.step0 + (unsigned long long)k;
+        if (k == 0 || (t & 1ull) == 0ull) words = action_words(r.seed_lo, r.seed_hi, env_global, L.i, t);
+        io.act = action_from_words(words, t);
+        if (r.action_out != nullptr && L.valid) st_stream((r.action_out + io.km) + L.m, io.act);
+      }
+      step_core<NT>(a, ws, L, io);
+    }
+    store_uav(a.s, L, io.cur, true);
+    if (L.valid & (L.i == 0)) a.s.steps[L.env] = io.steps;
   }
-  store_uav(a.s, L, io.cur, true);
-  if (L.valid & (L.i == 0)) a.s.steps[L.env] = io.steps;
 }
 
 // Resident CTAs per SM of the rollout kernel (measured on B200, profiles/r2_rollout_minb.md: 8 CTAs x 64 registers beats
@@ -361,7 +419,7 @@ template <int NT, int KIND>
 __global__ void __launch_bounds__(kThreads, UAVCA_ROLLOUT_MINB) rollout_multi_kernel(const __grid_constant__ KernelArgs a,
                                                                                   const __grid_constant__ RolloutArgs r) {
   __shared__ __align__(16) float smem[kWarpsPerBlock * kScratchFloats];
-  __shared__ __align__(16) float2 act_smem[kWarpsPerBlock * 64];  // per warp: two slots of 32 float2 actions
+  __shared__ __align__(512) float2 act_smem[kWarpsPerBlock * 64];  // per warp: two slots of 32 float2 actions
   const WarpScratch ws = warp_scratch(smem);
   const int warp_global = blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
   const int N = NT > 0 ? NT : a.N;
@@ -1163,15 +1221,19 @@ cudaError_t launch_rollout_multi(const KernelArgs& a, const RolloutArgs& r, cuda
   }
   const int grid = multi_grid(a.B, a.N);
   const bool block = r.action_block != nullptr;
-  // the plain instance (RolloutIO): the action mode the plain call implies — cartesian block actions, Philox actions
-  // scaled to the action box — and none of the optional outputs or accumulators
+  // the plain instance (PlainRolloutIO): the action mode the plain call implies — cartesian block actions, Philox actions
+  // scaled to the action box — and none of the optional outputs or accumulators.  Its step offsets are 32-bit: every
+  // element offset of the launch's blocks, up to the observations' K * M * 10, must stay below 2^31.
   const bool plain = a.io.final_obs == nullptr && a.io.reset_mask == nullptr && !a.c.track_scores &&
                      (block ? a.io.action_mode == UAVCA_ACTION_CARTESIAN
-                            : a.io.action_mode == UAVCA_ACTION_SCALED && r.action_out == nullptr);
+                            : a.io.action_mode == UAVCA_ACTION_SCALED && r.action_out == nullptr) &&
+                     (long long)r.K * r.M * UAVCA_OBS_DIM_MULTI < (1ll << 31);
+  RolloutArgs rp = r;
+  rp.KM = plain ? (unsigned)(r.K * r.M) : 0u;
   if (block && plain) {
-    UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT, kRolloutPlainBlock>, grid, st, a, r)));
+    UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT, kRolloutPlainBlock>, grid, st, a, rp)));
   } else if (plain) {
-    UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT, kRolloutPlainPhilox>, grid, st, a, r)));
+    UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT, kRolloutPlainPhilox>, grid, st, a, rp)));
   } else {
     UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT, kRolloutGeneral>, grid, st, a, r)));
   }

@@ -272,11 +272,12 @@ __device__ __forceinline__ ObsTail obs_tail(const Consts& c, float dx1, float dy
   const float2 nth = make_float2(-th_u, -th_u);
   const float2 v1 = wrap_units2(__ffma2_rn(b, make_float2(c.inv_pi, c.inv_pi), nth));  // bearings relative to the heading
   const float2 v2 = wrap_units2(__fadd2_rn(make_float2(h1, h2), nth));                 // neighbour headings, relative
+  const float2 d = __fmul2_rn(make_float2(sqrt_approx(s1), sqrt_approx(s2)), make_float2(c.inv_dsense, c.inv_dsense));
   ObsTail o;
-  o.a.x = have1 ? sqrt_approx(s1) * c.inv_dsense : 1.0f;  // :77
+  o.a.x = have1 ? d.x : 1.0f;                             // :77
   o.a.y = have1 ? v1.x : 1.0f;                            // :78-81 (no neighbour: bearing pi)
   o.b.x = have1 ? v2.x : 0.0f;                            // :82-85
-  o.b.y = have2 ? sqrt_approx(s2) * c.inv_dsense : 1.0f;  // :87
+  o.b.y = have2 ? d.y : 1.0f;                             // :87
   o.c.x = have2 ? v1.y : 1.0f;                            // :88-91
   o.c.y = have2 ? v2.y : 0.0f;                            // :92-95
   return o;
@@ -395,11 +396,12 @@ __device__ __forceinline__ ObsTail neighbours_mixed(const Consts& c, const WarpS
   const int slot = 2 * L.base + L.i;
   const float4 q1 = ws.ring()[slot + k1], q2 = ws.ring()[slot + k2];
   const float h1 = ws.ring_th()[slot + k1], h2 = ws.ring_th()[slot + k2];
-  const float dx1 = __fsub_rn(q1.y, px), dy1 = __fsub_rn(q1.w, py), dx2 = __fsub_rn(q2.y, px), dy2 = __fsub_rn(q2.w, py);
-  const float s1 = sq32(dx1, dy1), s2 = sq32(dx2, dy2);
-  const bool have1 = (k1 != 0) & (s1 < c.s_dsense_lt);
-  const bool have2 = have1 & (k2 != 0) & (s2 < c.s_dsense_lt);
-  return obs_tail(c, dx1, dy1, dx2, dy2, s1, s2, h1, h2, have1, have2, th_u);
+  // both neighbours at once on the packed FP32 pipe, each element exactly as __fsub_rn / sq32 (see dist2 of pair_scan_mixed)
+  const float2 dx = __fadd2_rn(make_float2(q1.y, q2.y), make_float2(-px, -px)), dy = __fadd2_rn(make_float2(q1.w, q2.w), make_float2(-py, -py));
+  const float2 zero = make_float2(0.f, 0.f), s = __fadd2_rn(__ffma2_rn(dx, dx, zero), __ffma2_rn(dy, dy, zero));
+  const bool have1 = (k1 != 0) & (s.x < c.s_dsense_lt);
+  const bool have2 = have1 & (k2 != 0) & (s.y < c.s_dsense_lt);
+  return obs_tail(c, dx.x, dy.x, dx.y, dy.y, s.x, s.y, h1, h2, have1, have2, th_u);
 }
 
 // Both pairwise passes of a step (or just the observation pass of a state at rest: old == new) for this lane's UAV:
@@ -433,8 +435,12 @@ struct Own {
 };
 __device__ __forceinline__ Own own_features(const Consts& c, float px, float py, float tx, float ty, double vx, double vy) {
   Own w;
-  const float tdx = __fsub_rn(tx, px), tdy = __fsub_rn(ty, py);
-  w.ssq = sq32(tdx, tdy);
+  // the two differences and the two squares on the packed FP32 pipe, each element exactly as __fsub_rn / sq32 (the
+  // squares as FFMA2 with a +0 addend, see pair_scan; a square is never -0)
+  const float2 td = __fadd2_rn(make_float2(tx, ty), make_float2(-px, -py));
+  const float tdx = td.x, tdy = td.y;
+  const float2 tsq = __ffma2_rn(td, td, make_float2(0.f, 0.f));
+  w.ssq = __fadd_rn(tsq.x, tsq.y);
   w.dist = __fsqrt_rn(w.ssq);
   w.vsq = sq64(vx, vy);
   const float fvx = (float)vx, fvy = (float)vy;
@@ -512,6 +518,49 @@ __device__ __forceinline__ void flush_warp_rows(const float* stage, float* g, co
     for (int r = 0; r < 5; ++r) {
       const int k = L.lane + 32 * r;
       if (k < n2) st_stream(g2 + k, s2[k]);
+    }
+  }
+}
+// The same stage by its shared-memory address (a 32-bit register computed once, where a loop would otherwise rebuild the
+// generic pointer from the thread index every step)
+__device__ __forceinline__ void sts_float2(unsigned smem_dst, float2 v) {
+  asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(smem_dst), "f"(v.x), "f"(v.y) : "memory");
+}
+__device__ __forceinline__ float2 lds_float2(unsigned smem_src) {
+  float2 v;
+  asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(smem_src) : "memory");
+  return v;
+}
+__device__ __forceinline__ float4 lds_float4(unsigned smem_src) {
+  float4 v;
+  asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(smem_src) : "memory");
+  return v;
+}
+__device__ __forceinline__ void stage_own(unsigned stage, int lane, float2 o01, float2 o23) {
+  const unsigned row = stage + lane * 40;
+  sts_float2(row, o01); sts_float2(row + 8, o23);
+}
+__device__ __forceinline__ void stage_neighbours(unsigned stage, int lane, const ObsTail& n) {
+  const unsigned row = stage + lane * 40;
+  sts_float2(row + 16, n.a); sts_float2(row + 24, n.b); sts_float2(row + 32, n.c);
+}
+__device__ __forceinline__ void flush_warp_rows(unsigned stage, float* g, const Lane& L) {
+  const int n2 = L.valid_lanes * 5;
+  if ((L.lanes_used & 1) == 0) {
+    const int n4 = n2 >> 1;
+    float4* g4 = reinterpret_cast<float4*>(g);
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+      const int k = L.lane + 32 * r;
+      if (k < n4) st_stream(g4 + k, lds_float4(stage + k * 16));
+    }
+    if ((n2 & 1) && L.lane == 0) st_stream(reinterpret_cast<float2*>(g) + (n2 - 1), lds_float2(stage + (n2 - 1) * 8));
+  } else {
+    float2* g2 = reinterpret_cast<float2*>(g);
+#pragma unroll
+    for (int r = 0; r < 5; ++r) {
+      const int k = L.lane + 32 * r;
+      if (k < n2) st_stream(g2 + k, lds_float2(stage + k * 8));
     }
   }
 }
