@@ -190,7 +190,7 @@ struct uavca_handle {
   uavca_layout pool_layout{};
   double4* ring64 = nullptr;  // reset(circular=True) table (owned): per UAV (pos.x, pos.y, tgt.x, tgt.y) in float64
   long long launches = 0;
-  int path = UAVCA_PATH_LANES;  // UAVCA_STEP_PATH=tma in the environment selects the bulk (TMA) kernel for whole tiles (A/B measurements)
+  bool cta_pack = true;  // UAVCA_STEP_PATH=plain in the environment keeps every N <= 32 on the one-env-per-warp step kernel
   // end-to-end (host buffer) path, created lazily
   static constexpr int kHostStreams = 3;
   static constexpr int kChunks = 8;
@@ -300,11 +300,7 @@ int uavca_create(const uavca_config* cfg, int device, uavca_handle** out) {
   h->consts = derive_consts(*cfg);
   h->device = device;
   compute_layout(cfg->num_envs, cfg->num_agents, cfg->kind == UAVCA_KIND_MULTI && cfg->circular, &h->layout);
-  if (const char* p = std::getenv("UAVCA_STEP_PATH")) {  // A/B measurements: tma | prefetch (always) | plain (never prefetch)
-    h->path = std::strcmp(p, "tma") == 0 ? UAVCA_PATH_AUTO
-              : std::strcmp(p, "prefetch") == 0 ? UAVCA_PATH_PREFETCH
-              : std::strcmp(p, "plain") == 0 ? UAVCA_PATH_PLAIN : UAVCA_PATH_LANES;
-  }
+  if (const char* p = std::getenv("UAVCA_STEP_PATH")) h->cta_pack = std::strcmp(p, "plain") != 0;
   if (cfg->kind == UAVCA_KIND_MULTI && cfg->circular) {
     // multi_uav_world_2d.py:157-163 with the HOST libm: the reference evaluates math.cos / math.sin (glibc) in float64,
     // and the device's cos / sin are not bit-identical to it; the ring is a table of N entries computed once here
@@ -413,9 +409,8 @@ int uavca_step_multi(uavca_handle* h, void* state, const float* action, int acti
   a.io.action = reinterpret_cast<const float2*>(action);
   a.io.obs = obs; a.io.reward = reward; a.io.done = done; a.io.final_obs = final_obs; a.io.reset_mask = reset_mask;
   a.io.action_mode = action_mode; a.io.evaluate = evaluate;
-  int launched = 0;
-  cudaError_t e = launch_step_multi(a, (cudaStream_t)stream, &launched, h->path);
-  h->launches += launched;
+  cudaError_t e = launch_step_multi(a, (cudaStream_t)stream, h->cta_pack);
+  h->launches += 1;
   if (e != cudaSuccess) return fail_cuda("uavca_step_multi", e);
   return 0;
 }
@@ -453,14 +448,13 @@ int uavca_step_f64(uavca_handle* h, void* state, const double* action, int evalu
   a.io.obs = obs; a.io.reward = reward; a.io.done = done; a.io.final_obs = final_obs; a.io.reset_mask = reset_mask;
   a.io.action_mode = UAVCA_ACTION_CARTESIAN; a.io.evaluate = evaluate;
   cudaError_t e;
-  int launched = 1;
   if (h->cfg.kind == UAVCA_KIND_SINGLE) {
     a.io.distance = distance;
     e = launch_step_single(a, (cudaStream_t)stream);
   } else {
-    e = launch_step_multi(a, (cudaStream_t)stream, &launched, h->path);  // the general one-thread-per-env kernel
+    e = launch_step_multi(a, (cudaStream_t)stream, h->cta_pack);  // the general one-thread-per-env kernel
   }
-  h->launches += launched;
+  h->launches += 1;
   if (e != cudaSuccess) return fail_cuda("uavca_step_f64", e);
   return 0;
 }
@@ -556,9 +550,8 @@ int uavca_step_host(uavca_handle* h, void* state, const float* host_action, int 
     a.io.done = reinterpret_cast<uint8_t*>(m_done);
     a.io.action_mode = action_mode; a.io.evaluate = evaluate;
     cudaStream_t st = caller;
-    int launched = 1;
-    e = h->cfg.kind == UAVCA_KIND_SINGLE ? launch_step_single(a, st) : launch_step_multi(a, st, &launched, h->path);
-    h->launches += launched;
+    e = h->cfg.kind == UAVCA_KIND_SINGLE ? launch_step_single(a, st) : launch_step_multi(a, st, h->cta_pack);
+    h->launches += 1;
     if (e != cudaSuccess) return fail_cuda("uavca_step_host launch", e);
     if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return fail_cuda("stream synchronize", e);
     return 0;
@@ -593,9 +586,8 @@ int uavca_step_host(uavca_handle* h, void* state, const float* host_action, int 
       a.io.action = reinterpret_cast<const float2*>(h->d_action + m0 * 2);
       a.io.obs = h->d_obs + m0 * D; a.io.reward = h->d_reward + m0; a.io.done = h->d_done + m0;
       a.io.action_mode = action_mode; a.io.evaluate = evaluate;
-      int launched = 1;
-      e = h->cfg.kind == UAVCA_KIND_SINGLE ? launch_step_single(a, s_in) : launch_step_multi(a, s_in, &launched, h->path);
-      h->launches += launched;
+      e = h->cfg.kind == UAVCA_KIND_SINGLE ? launch_step_single(a, s_in) : launch_step_multi(a, s_in, h->cta_pack);
+      h->launches += 1;
       if (e != cudaSuccess) return fail_cuda("uavca_step_host launch", e);
       if ((e = cudaEventRecord(h->chunk_done[k], s_in)) != cudaSuccess) return fail_cuda("event record", e);
       if ((e = cudaStreamWaitEvent(s_out, h->chunk_done[k], 0)) != cudaSuccess) return fail_cuda("stream wait", e);
@@ -626,9 +618,8 @@ int uavca_step_host(uavca_handle* h, void* state, const float* host_action, int 
     a.io.action = reinterpret_cast<const float2*>(h->d_action + m0 * 2);
     a.io.obs = h->d_obs + m0 * D; a.io.reward = h->d_reward + m0; a.io.done = h->d_done + m0;
     a.io.action_mode = action_mode; a.io.evaluate = evaluate;
-    int launched = 1;
-    e = h->cfg.kind == UAVCA_KIND_SINGLE ? launch_step_single(a, st) : launch_step_multi(a, st, &launched, h->path);
-    h->launches += launched;
+    e = h->cfg.kind == UAVCA_KIND_SINGLE ? launch_step_single(a, st) : launch_step_multi(a, st, h->cta_pack);
+    h->launches += 1;
     if (e != cudaSuccess) return fail_cuda("uavca_step_host launch", e);
     if ((e = cudaMemcpyAsync(host_obs + m0 * D, h->d_obs + m0 * D, mc * D * sizeof(float), cudaMemcpyDeviceToHost, st)) != cudaSuccess)
       return fail_cuda("D2H obs", e);
@@ -681,9 +672,8 @@ int uavca_rollout(uavca_handle* h, void* state, int32_t K, const float* action_b
       a.io.done = done + (size_t)k * M;
       a.io.final_obs = final_obs ? final_obs + (size_t)k * M * UAVCA_OBS_DIM_MULTI : nullptr;
       a.io.reset_mask = reset_mask ? reset_mask + (size_t)k * h->cfg.num_envs : nullptr;
-      int launched = 0;
-      cudaError_t e = launch_step_multi(a, st, &launched, h->path);
-      h->launches += launched;
+      cudaError_t e = launch_step_multi(a, st, h->cta_pack);
+      h->launches += 1;
       if (e != cudaSuccess) return fail_cuda("uavca_rollout", e);
     }
     return 0;

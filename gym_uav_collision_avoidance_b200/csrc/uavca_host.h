@@ -7,10 +7,9 @@
 
 namespace uavca {
 
-// path: which kernel(s) may run the step (UAVCA_PATH_AUTO: TMA bulk kernel for whole tiles + per-lane kernel for the
-// ragged rest; UAVCA_PATH_LANES: per-lane kernel only).  *launched receives the number of kernels launched.
-enum : int { UAVCA_PATH_AUTO = 0, UAVCA_PATH_LANES = 1, UAVCA_PATH_PREFETCH = 2, UAVCA_PATH_PLAIN = 3 };
-cudaError_t launch_step_multi(const KernelArgs& a, cudaStream_t st, int* launched, int path);
+// One kernel per call when B > 0.  cta_pack: envs of 11 and 17..25 UAVs run on the CTA-packed kernel (uavca_cta.cuh);
+// false keeps them on the one-env-per-warp kernel.
+cudaError_t launch_step_multi(const KernelArgs& a, cudaStream_t st, bool cta_pack);
 cudaError_t launch_step_multi_ring(const KernelArgs& a, const RingSink& g, cudaStream_t st);
 cudaError_t launch_rollout_multi(const KernelArgs& a, const RolloutArgs& r, cudaStream_t st);
 cudaError_t launch_rollout_single(const KernelArgs& a, const RolloutArgs& r, cudaStream_t st);

@@ -9,15 +9,12 @@
 // streaming accesses; neighbour interaction stays on chip (per-warp shared-memory ring, uavca_multi.cuh).  No tensor
 // cores: there is no dense contraction anywhere in the step.  (The fused policy kernel, which is GEMM-shaped, lives
 // in uavca_policy.cu.)
-#include <atomic>
 #include <cmath>
-#include <cstdlib>
 
 #include "uavca_host.h"
 #include "uavca_multi.cuh"
 #include "uavca_seq.cuh"
 #include "uavca_cta.cuh"
-#include "uavca_tma.cuh"
 
 namespace uavca {
 
@@ -25,7 +22,7 @@ namespace uavca {
 // Multi-UAV world
 // ================================================================================================================
 
-// I/O policy of step_core for per-lane streaming global accesses (ragged tails, unaligned tensors, any N).
+// I/O policy of step_core for per-lane streaming global accesses (any N, ragged last warp).
 struct GlobalIO {
   const KernelArgs& a;
   const Lane& L;
@@ -440,100 +437,6 @@ __global__ void __launch_bounds__(kThreads) sample_actions_kernel(const __grid_c
   out[m] = action_from_words(action_words(seed_lo, seed_hi, c.env_base + env, i, t), t);
 }
 
-// ---- persistent variant with cp.async input prefetch (large batches) ----------------------------------------------------
-// ncu on step_multi_kernel<32> (profiles/r2_full_c4_step_multi_n32.md): a fifth of the warp-time is spent waiting for
-// the warp's own state to arrive (long scoreboard on the first use of the loads).  Here every warp walks warp-tiles
-// w, w + G, w + 2G, ...; while it computes one tile, the next tile's state and actions are already on their way INTO
-// SHARED MEMORY (cp.async / LDGSTS: no registers held, unlike a register prefetch).  Same step_core, same outputs.
-// MEASURED (profiles/r2_prefetch_variant.md): the long-scoreboard stall disappears (2.05 -> 0.16 warps per issue cycle)
-// but issue utilisation does not rise (76.5 % -> 72.5 %): the idle issue slots come from the dependent integer min/max
-// chains and ALU-pipe contention, not from load latency, and the hardware CTA scheduler already overlaps one CTA's loads
-// with its neighbours' compute.  151.6 vs 132.3 us at N=32, B=131,072 — slower everywhere, hence opt-in only
-// (UAVCA_STEP_PATH=prefetch), parity-tested.
-constexpr int kPfStageBytes = 32 * (16 + 8 + 8 + 8 + 4 + 4);  // vel, pos, tgt, action, init, prev of one warp-tile
-
-
-struct PfStage {
-  double2* vel;
-  float2 *pos, *tgt, *act;
-  float *init, *prev;
-};
-__device__ __forceinline__ PfStage pf_stage(unsigned char* base) {
-  PfStage st;
-  st.vel = reinterpret_cast<double2*>(base);
-  st.pos = reinterpret_cast<float2*>(base + 32 * 16);
-  st.tgt = st.pos + 32;
-  st.act = st.tgt + 32;
-  st.init = reinterpret_cast<float*>(st.act + 32);
-  st.prev = st.init + 32;
-  return st;
-}
-
-struct PfIO : GlobalIO {
-  Uav pre;
-  float2 act;
-  int steps;
-  __device__ __forceinline__ Uav load_uav() const { return pre; }
-  __device__ __forceinline__ float2 load_action() const { return act; }
-  __device__ __forceinline__ int load_steps() const { return steps; }
-  __device__ __forceinline__ void loads_done() const {}
-};
-
-template <int NT>
-__global__ void __launch_bounds__(kThreads, kMinBlocksPerSM) step_multi_pf_kernel(const __grid_constant__ KernelArgs a,
-                                                                                  const int num_tiles) {
-  __shared__ __align__(16) float smem[kWarpsPerBlock * kScratchFloats];
-  __shared__ __align__(16) unsigned char stage_mem[kWarpsPerBlock * kPfStageBytes];
-  const WarpScratch ws = warp_scratch(smem);
-  const PfStage st = pf_stage(stage_mem + (threadIdx.x >> 5) * kPfStageBytes);
-  const int lane = threadIdx.x & 31;
-  const int stride = gridDim.x * kWarpsPerBlock;
-  int wt = blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
-  cudaGridDependencySynchronize();
-  if (wt >= num_tiles) return;
-  // every tile of this kernel is a FULL warp-tile (the launcher hands the ragged rest to the per-lane kernel)
-  unsigned nflags = 0u;
-  int nsteps = 0;
-  auto prefetch = [&](int tile) {
-    const Lane P = make_lane<NT, true>(a.B, a.N, tile);
-    if (P.valid) {
-      cp_async(st.vel + lane, a.s.vel + P.m, 16);
-      cp_async(st.pos + lane, a.s.pos + P.m, 8);
-      cp_async(st.tgt + lane, a.s.tgt + P.m, 8);
-      cp_async(st.act + lane, a.io.action + P.m, 8);
-      cp_async(st.init + lane, a.s.init + P.m, 4);
-      cp_async(st.prev + lane, a.s.prev + P.m, 4);
-      nflags = ld_stream(a.s.flags + P.m);  // one register each: consumed only at the top of the next tile
-      nsteps = a.s.steps[P.env];
-    }
-  };
-  prefetch(wt);
-  cudaTriggerProgrammaticLaunchCompletion();
-  while (true) {
-    const Lane L = make_lane<NT, true>(a.B, a.N, wt);
-    cp_async_wait_all();
-    __syncwarp();
-    PfIO io{{a, L, ws.stage}, Uav{}, make_float2(0.f, 0.f), 0};
-    if (L.valid) {
-      const double2 v = st.vel[lane];
-      const float2 p = st.pos[lane], t = st.tgt[lane];
-      io.pre.px = p.x; io.pre.py = p.y; io.pre.tx = t.x; io.pre.ty = t.y; io.pre.vx = v.x; io.pre.vy = v.y;
-      io.pre.init = st.init[lane]; io.pre.prev = st.prev[lane]; io.pre.flags = nflags;
-      io.act = st.act[lane];
-      io.steps = nsteps;
-    } else {  // idle lanes (32 is not a multiple of N): a harmless UAV in ordinary flight, as in load_uav()
-      io.pre.px = io.pre.py = io.pre.ty = 0.f; io.pre.tx = 8.f; io.pre.init = io.pre.prev = 8.f;
-      io.pre.vx = 1.0; io.pre.vy = 0.0; io.pre.flags = 0u;
-    }
-    __syncwarp();  // the stage has been read out: refill it for the next tile while this one is computed
-    const int next = wt + stride;
-    if (next < num_tiles) prefetch(next);
-    step_core<NT>(a, ws, L, io);
-    if (next >= num_tiles) break;
-    wt = next;
-  }
-}
-
 template <int NT>
 __global__ void __launch_bounds__(kThreads) reset_multi_kernel(const __grid_constant__ KernelArgs a, const uint8_t* mask) {
   __shared__ __align__(16) float smem[kWarpsPerBlock * kScratchFloats];
@@ -933,10 +836,9 @@ static inline int multi_grid(int B, int N) {
     default: { constexpr int NT = 0; CALL; } break;  \
   }
 
-// The step kernel is launched with programmatic stream serialization (PDL): its blocks may become resident while
-// the previous kernel in the stream drains, and wait in cudaGridDependencySynchronize() before touching memory.
-template <int NT>
-static cudaError_t launch_step_multi_n(const KernelArgs& a, int grid, cudaStream_t st) {
+// PDL: the kernel's CTAs may become resident while the previous kernel in the stream drains (DESIGN §5)
+template <typename... P, typename... A>
+static cudaError_t launch_pdl(void (*kernel)(P...), int grid, cudaStream_t st, const A&... args) {
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(kThreads);
@@ -947,240 +849,30 @@ static cudaError_t launch_step_multi_n(const KernelArgs& a, int grid, cudaStream
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, step_multi_kernel<NT>, a);
+  return cudaLaunchKernelEx(&cfg, kernel, args...);
 }
-
-// ---- bulk path (uavca_tma.cuh): persistent grid sized to the SM slots the kernel can hold --------------------------
-
-template <typename Kernel>
-static cudaError_t launch_pdl(Kernel kernel, int grid, int threads, size_t smem, cudaStream_t st, const KernelArgs& a,
-                              int num_tiles) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(threads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, a, num_tiles);
-}
-
-template <int NT, bool FINAL>
-static cudaError_t launch_step_tma_n(const KernelArgs& a, int num_tiles, cudaStream_t st) {
-  using G = TmaGeom<NT, FINAL>;
-  constexpr int kMaxDev = 64;
-  static std::atomic<int> slots[kMaxDev];  // resident CTAs per device for this instantiation (0 = not configured yet)
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) return e;
-  if (dev < 0 || dev >= kMaxDev) return cudaErrorInvalidDevice;
-  auto kernel = step_multi_tma_kernel<NT, FINAL>;
-  if (slots[dev] == 0) {
-    e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM_BYTES);
-    if (e != cudaSuccess) return e;
-    int per_sm = 0, sms = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, G::THREADS, G::SMEM_BYTES);
-    if (e != cudaSuccess) return e;
-    e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) return cudaErrorLaunchOutOfResources;
-    slots[dev] = per_sm * sms;
-  }
-  const int n_slots = slots[dev];
-  const int grid = num_tiles < n_slots ? num_tiles : n_slots;
-  return launch_pdl(kernel, grid, G::THREADS, G::SMEM_BYTES, st, a, num_tiles);
-}
-
-// envs per tile of the bulk path for this N (0: no bulk path, the per-lane kernel takes everything)
-static int tma_tile_envs(int N) {
-  switch (N) {
-    case 2: return TmaGeom<2, false>::E;
-    case 4: return TmaGeom<4, false>::E;
-    case 5: return TmaGeom<5, false>::E;
-    case 8: return TmaGeom<8, false>::E;
-    case 10: return TmaGeom<10, false>::E;
-    case 16: return TmaGeom<16, false>::E;
-    case 32: return TmaGeom<32, false>::E;
-    default: return 0;
-  }
-}
-
-#define UAVCA_DISPATCH_TMA(N, CALL)                  \
-  switch (N) {                                       \
-    case 2: { constexpr int NT = 2; CALL; } break;   \
-    case 4: { constexpr int NT = 4; CALL; } break;   \
-    case 5: { constexpr int NT = 5; CALL; } break;   \
-    case 8: { constexpr int NT = 8; CALL; } break;   \
-    case 10: { constexpr int NT = 10; CALL; } break; \
-    case 16: { constexpr int NT = 16; CALL; } break; \
-    case 32: { constexpr int NT = 32; CALL; } break; \
-    default: break;                                  \
-  }
-
-static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-
-// persistent prefetching kernel: grid = resident CTA slots of the device
-template <int NT>
-static cudaError_t launch_step_pf_n(const KernelArgs& a, int num_tiles, cudaStream_t st) {
-  constexpr int kMaxDev = 64;
-  static std::atomic<int> slots[kMaxDev];
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) return e;
-  if (dev < 0 || dev >= kMaxDev) return cudaErrorInvalidDevice;
-  auto kernel = step_multi_pf_kernel<NT>;
-  if (slots[dev] == 0) {
-    int per_sm = 0, sms = 0;
-    cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, 0);
-    if (e != cudaSuccess) return e;
-    e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) return cudaErrorLaunchOutOfResources;
-    slots[dev] = per_sm * sms;
-  }
-  const int ctas = (num_tiles + kWarpsPerBlock - 1) / kWarpsPerBlock;
-  const int n_slots = slots[dev];
-  return launch_pdl(kernel, ctas < n_slots ? ctas : n_slots, kThreads, 0, st, a, num_tiles);
-}
-
 
 // the general one-thread-per-env kernels (uavca_seq.cuh) serve the float64 world and envs wider than a warp
 static inline bool wants_seq(const KernelArgs& a) { return a.c.circular != 0 || a.N > 32; }
 
-template <int NT>
-static cudaError_t launch_step_multi_f64_n(const KernelArgs& a, int grid, cudaStream_t st) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = 0;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, step_multi_f64_kernel<NT>, a);
-}
-
-cudaError_t launch_step_multi(const KernelArgs& a, cudaStream_t st, int* launched, int path) {
-  if (launched) *launched = 0;
+cudaError_t launch_step_multi(const KernelArgs& a, cudaStream_t st, bool cta_pack) {
   if (a.B <= 0) return cudaSuccess;
   cudaError_t e = cudaSuccess;
   if (wants_seq(a)) {
     if (a.c.circular) step_multi_seq_kernel<double><<<flat_grid(a.B), kThreads, 0, st>>>(a);
     else step_multi_seq_kernel<float><<<flat_grid(a.B), kThreads, 0, st>>>(a);
-    if (launched) *launched = 1;
-    return cudaGetLastError();
-  }
-  if (a.io.action64 != nullptr) {  // float64 actions: the warp kernel fed by GlobalIO64
-    UAVCA_DISPATCH_N(a.N, (e = launch_step_multi_f64_n<NT>(a, multi_grid(a.B, a.N), st)));
-    if (e != cudaSuccess) return e;
-    if (launched) *launched = 1;
-    return cudaGetLastError();
-  }
-  if (cta_packs(a.N, false) && path != UAVCA_PATH_PLAIN && path != UAVCA_PATH_PREFETCH && path != UAVCA_PATH_AUTO) {
+  } else if (a.io.action64 != nullptr) {  // float64 actions: the warp kernel fed by GlobalIO64
+    UAVCA_DISPATCH_N(a.N, (e = launch_pdl(step_multi_f64_kernel<NT>, multi_grid(a.B, a.N), st, a)));
+  } else if (cta_pack && cta_packs(a.N, false)) {
     // 17..25 UAVs per env: 5..7 envs packed across the 4 warps of a CTA instead of one env per warp (uavca_cta.cuh).
     // Measured (B*N = 2 Mi UAVs, one stream): N=17 98 vs 136 us, N=20 101 vs 122, N=24 107 vs 113; from N=26 a CTA
     // holds 4 envs like 4 warps do and the barriers only cost (N=28 119 vs 108 us), so those stay on the warp kernel.
     const int envs_per_cta = kThreads / a.N;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((a.B + envs_per_cta - 1) / envs_per_cta);
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = 0;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    e = cudaLaunchKernelEx(&cfg, step_multi_cta_kernel, a);
-    if (e != cudaSuccess) return e;
-    if (launched) *launched = 1;
-    return cudaGetLastError();
+    e = launch_pdl(step_multi_cta_kernel, (a.B + envs_per_cta - 1) / envs_per_cta, st, a);
+  } else {
+    UAVCA_DISPATCH_N(a.N, (e = launch_pdl(step_multi_kernel<NT>, multi_grid(a.B, a.N), st, a)));
   }
-  if (path == UAVCA_PATH_PREFETCH) {
-    // opt-in (UAVCA_STEP_PATH=prefetch; measured slower than the per-lane kernel at every size, DESIGN.md 6.3): whole
-    // warp-tiles go through the persistent cp.async-prefetch kernel, the ragged rest through the per-lane kernel
-    const int epw = 32 / a.N;
-    const int full_tiles = a.B / epw;
-    if (full_tiles > 0 && aligned16(a.s.vel) && aligned16(a.s.pos) && aligned16(a.s.tgt) && aligned16(a.io.action)) {
-      UAVCA_DISPATCH_N(a.N, (e = launch_step_pf_n<NT>(a, full_tiles, st)));
-      if (e != cudaSuccess) return e;
-      if (launched) *launched += 1;
-      const int done_envs = full_tiles * epw;
-      if (done_envs < a.B) {
-        KernelArgs r = a;
-        const long long m0 = (long long)done_envs * a.N;
-        r.s = offset_view(a.s, done_envs, a.N);
-        r.c.env_base += done_envs;
-        r.B = a.B - done_envs;
-        r.io.action += m0;
-        r.io.obs += m0 * UAVCA_OBS_DIM_MULTI;
-        r.io.reward += m0;
-        r.io.done += m0;
-        if (r.io.final_obs) r.io.final_obs += m0 * UAVCA_OBS_DIM_MULTI;
-        if (r.io.reset_mask) r.io.reset_mask += done_envs;
-        UAVCA_DISPATCH_N(r.N, (e = launch_step_multi_n<NT>(r, multi_grid(r.B, r.N), st)));
-        if (e != cudaSuccess) return e;
-        if (launched) *launched += 1;
-      }
-      return cudaGetLastError();
-    }
-  }
-  // whole tiles go through the bulk (TMA) kernel, the ragged rest through the per-lane kernel
-  int tile_envs = path == UAVCA_PATH_AUTO ? tma_tile_envs(a.N) : 0;
-  if (tile_envs && !(aligned16(a.io.action) && aligned16(a.io.obs) && aligned16(a.io.reward) && aligned16(a.io.done) &&
-                     aligned16(a.io.final_obs) && aligned16(a.s.pos) && aligned16(a.s.vel) && aligned16(a.s.tgt) &&
-                     aligned16(a.s.init) && aligned16(a.s.prev) && aligned16(a.s.flags) && aligned16(a.s.steps)))
-    tile_envs = 0;
-  const int tiles = tile_envs ? a.B / tile_envs : 0;
-  const int bulk_envs = tiles * tile_envs;
-  if (tiles > 0) {
-    if (a.io.final_obs) {
-      UAVCA_DISPATCH_TMA(a.N, (e = launch_step_tma_n<NT, true>(a, tiles, st)));
-    } else {
-      UAVCA_DISPATCH_TMA(a.N, (e = launch_step_tma_n<NT, false>(a, tiles, st)));
-    }
-    if (e != cudaSuccess) return e;
-    if (launched) *launched += 1;
-  }
-  if (bulk_envs < a.B) {
-    KernelArgs r = a;
-    const long long m0 = (long long)bulk_envs * a.N;
-    r.s = offset_view(a.s, bulk_envs, a.N);
-    r.c.env_base += bulk_envs;
-    r.B = a.B - bulk_envs;
-    r.io.action += m0;
-    r.io.obs += m0 * UAVCA_OBS_DIM_MULTI;
-    r.io.reward += m0;
-    r.io.done += m0;
-    if (r.io.final_obs) r.io.final_obs += m0 * UAVCA_OBS_DIM_MULTI;
-    if (r.io.reset_mask) r.io.reset_mask += bulk_envs;
-    const int grid = multi_grid(r.B, r.N);
-    UAVCA_DISPATCH_N(r.N, (e = launch_step_multi_n<NT>(r, grid, st)));
-    if (e != cudaSuccess) return e;
-    if (launched) *launched += 1;
-  }
-  return cudaGetLastError();
-}
-
-template <int NT>
-static cudaError_t launch_step_multi_ring_n(const KernelArgs& a, const RingSink& g, int grid, cudaStream_t st) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = 0;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, step_multi_ring_kernel<NT>, a, g);
+  return e != cudaSuccess ? e : cudaGetLastError();
 }
 
 // step + replay append in one launch: the warp kernels only (N <= 32, float32 world)
@@ -1188,35 +880,18 @@ cudaError_t launch_step_multi_ring(const KernelArgs& a, const RingSink& g, cudaS
   if (a.B <= 0) return cudaSuccess;
   if (wants_seq(a)) return cudaErrorNotSupported;
   cudaError_t e = cudaSuccess;
-  UAVCA_DISPATCH_N(a.N, (e = launch_step_multi_ring_n<NT>(a, g, multi_grid(a.B, a.N), st)));
-  if (e != cudaSuccess) return e;
-  return cudaGetLastError();
-}
-
-template <typename Kernel>
-static cudaError_t launch_pdl2(Kernel kernel, int grid, cudaStream_t st, const KernelArgs& a, const RolloutArgs& r) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = 0;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, a, r);
+  UAVCA_DISPATCH_N(a.N, (e = launch_pdl(step_multi_ring_kernel<NT>, multi_grid(a.B, a.N), st, a, g)));
+  return e != cudaSuccess ? e : cudaGetLastError();
 }
 
 cudaError_t launch_rollout_multi(const KernelArgs& a, const RolloutArgs& r, cudaStream_t st) {
   if (a.B <= 0 || r.K <= 0) return cudaSuccess;
   cudaError_t e = cudaSuccess;
   // 17..25 UAVs per env: the CTA-packed kernel (5..7 envs on the 128 threads of a CTA instead of one env per warp), as in
-  // launch_step_multi; UAVCA_ROLLOUT_CTA=0 keeps the warp kernel (A/B measurements)
-  static const bool cta_ok = [] { const char* v = getenv("UAVCA_ROLLOUT_CTA"); return !(v && v[0] == '0'); }();
-  if (cta_ok && cta_packs(a.N, true)) {
+  // launch_step_multi
+  if (cta_packs(a.N, true)) {
     const int envs_per_cta = kThreads / a.N;
-    e = launch_pdl2(rollout_multi_cta_kernel, (a.B + envs_per_cta - 1) / envs_per_cta, st, a, r);
+    e = launch_pdl(rollout_multi_cta_kernel, (a.B + envs_per_cta - 1) / envs_per_cta, st, a, r);
     return e != cudaSuccess ? e : cudaGetLastError();
   }
   const int grid = multi_grid(a.B, a.N);
@@ -1231,18 +906,18 @@ cudaError_t launch_rollout_multi(const KernelArgs& a, const RolloutArgs& r, cuda
   RolloutArgs rp = r;
   rp.KM = plain ? (unsigned)(r.K * r.M) : 0u;
   if (block && plain) {
-    UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT, kRolloutPlainBlock>, grid, st, a, rp)));
+    UAVCA_DISPATCH_N(a.N, (e = launch_pdl(rollout_multi_kernel<NT, kRolloutPlainBlock>, grid, st, a, rp)));
   } else if (plain) {
-    UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT, kRolloutPlainPhilox>, grid, st, a, rp)));
+    UAVCA_DISPATCH_N(a.N, (e = launch_pdl(rollout_multi_kernel<NT, kRolloutPlainPhilox>, grid, st, a, rp)));
   } else {
-    UAVCA_DISPATCH_N(a.N, (e = launch_pdl2(rollout_multi_kernel<NT, kRolloutGeneral>, grid, st, a, r)));
+    UAVCA_DISPATCH_N(a.N, (e = launch_pdl(rollout_multi_kernel<NT, kRolloutGeneral>, grid, st, a, r)));
   }
   return e != cudaSuccess ? e : cudaGetLastError();
 }
 
 cudaError_t launch_rollout_single(const KernelArgs& a, const RolloutArgs& r, cudaStream_t st) {
   if (a.B <= 0 || r.K <= 0) return cudaSuccess;
-  const cudaError_t e = launch_pdl2(rollout_single_kernel, flat_grid(a.B), st, a, r);
+  const cudaError_t e = launch_pdl(rollout_single_kernel, flat_grid(a.B), st, a, r);
   return e != cudaSuccess ? e : cudaGetLastError();
 }
 

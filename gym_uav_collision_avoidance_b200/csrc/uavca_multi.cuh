@@ -652,9 +652,10 @@ __device__ __forceinline__ void reset_multi(const KernelArgs& a, const Lane& L, 
 
 // ================================================================================================================
 // The step itself, independent of where the state and the I/O live.  `IO` is a policy that moves one UAV's data:
-//   GlobalIO (uavca_kernels.cu)  per-lane streaming global loads/stores           (ragged tails, any N, any alignment)
-//   SmemIO   (uavca_tma.cuh)     shared-memory stage filled / drained by TMA bulk copies
-// Both run exactly this code, so they cannot disagree on semantics.
+//   GlobalIO / GlobalIO64 (uavca_kernels.cu)  per-lane streaming global loads/stores, float32 / float64 actions
+//   RingIO                (uavca_kernels.cu)  GlobalIO's outputs, and each transition appended to a device replay ring
+//   RolloutIO / PlainRolloutIO (uavca_kernels.cu)  state in registers for K steps, outputs to [K][...] blocks
+// All of them run exactly this code, so they cannot disagree on semantics.
 //
 //   Uav   load_uav();  float2 load_action();  int load_steps();        (load_steps: every lane, its env's counter)
 //   void  loads_done();                                                (every input of this warp is in registers)

@@ -167,10 +167,11 @@ def rollout_vs_oracle(cfg: O.Config, steps, seed, evaluate=False, crowd=None, nt
     return events, orc
 
 
-@pytest.mark.parametrize("n", [1, 2, 3, 4, 5, 7, 8, 9, 10, 11, 12, 13, 16, 17, 24, 31, 32])
-def test_multi_rollout_all_agent_counts(n):
-    """Every N in 1..32 maps to a different lane layout (specialised or generic kernel, ragged last warp)."""
-    B = 257  # not a multiple of any envs-per-warp: exercises the tail
+@pytest.mark.parametrize("n,B", [pytest.param(n, 257, id=str(n)) for n in [1, 2, 3, 4, 5, 7, 8, 9, 10, 11, 12, 13, 16, 17, 24, 31, 32]]
+                         + [(7, 1), (16, 3)])
+def test_multi_rollout_all_agent_counts(n, B):
+    """Every N in 1..32 maps to a different lane layout (specialised or generic kernel, ragged last warp).  B = 257 is not
+    a multiple of any envs-per-warp; B = 1 and B = 3 fill less than one CTA (a partial warp, then idle warps)."""
     cfg = O.multi_config(B, n, reset_mode=O.RESET_ON_DONE0, max_episode_steps=40, seed=1000 + n, x_size=24.0, y_size=24.0)
     ev, _ = rollout_vs_oracle(cfg, steps=120, seed=n, crowd=0.4)
     assert ev["resets"] > 0
@@ -365,49 +366,6 @@ def test_multi_c4_full_size_properties_and_window():
     assert float(d.min()) > 2.0 - 1e-6
     assert_state_equal_window = env.state.vel[sl].cpu().numpy()
     assert np.array_equal(assert_state_equal_window, orc.state.vel)
-
-
-def test_tma_variant_matches_the_oracle(monkeypatch):
-    """The opt-in bulk-copy kernel (UAVCA_STEP_PATH=tma: TMA loads/stores of whole tiles through an mbarrier ring,
-    ragged rest on the per-lane kernel) runs the same step_core and must give the same results."""
-    monkeypatch.setenv("UAVCA_STEP_PATH", "tma")
-    for n, B in ((8, 4099), (10, 2050), (32, 515), (5, 3000)):
-        cfg = O.multi_config(B, n, reset_mode=O.RESET_ON_DONE0, max_episode_steps=40, seed=60 + n)
-        ev, _ = rollout_vs_oracle(cfg, steps=60, seed=n, check_every=4)
-        assert ev["resets"] > 0
-
-
-def test_prefetch_variant_matches_the_oracle(monkeypatch):
-    """The persistent cp.async-prefetch kernel (taken automatically for large batches, forced here with
-    UAVCA_STEP_PATH=prefetch: whole warp-tiles prefetched into shared memory one tile ahead, ragged rest on the per-lane
-    kernel) runs the same step_core and must give the same results — including batches so small that most resident
-    warps get no tile, and batches where every warp walks several tiles."""
-    monkeypatch.setenv("UAVCA_STEP_PATH", "prefetch")
-    for n, B in ((8, 4099), (10, 2050), (32, 515), (5, 3000), (2, 70001), (32, 20000), (16, 3), (7, 1)):
-        cfg = O.multi_config(B, n, reset_mode=O.RESET_ON_DONE0, max_episode_steps=40, seed=160 + n)
-        ev, _ = rollout_vs_oracle(cfg, steps=60, seed=n, check_every=4)
-        assert ev["resets"] > 0 or B < 10
-
-
-def test_prefetch_variant_equals_the_plain_kernel_at_scale(monkeypatch):
-    """N=32, 262,144 envs (8.4 M UAVs: every resident warp walks ~55 tiles): prefetch kernel == per-lane kernel, bit for bit."""
-    G = _b200()
-    B, N = 262144, 32
-    kw = dict(num_agents=N, seed=77, reset_mode=O.RESET_ON_DONE0, max_episode_steps=9)
-    monkeypatch.setenv("UAVCA_STEP_PATH", "plain")
-    e1 = G.BatchedMultiUAVWorld2D(B, **kw)
-    monkeypatch.setenv("UAVCA_STEP_PATH", "prefetch")
-    e2 = G.BatchedMultiUAVWorld2D(B, **kw)
-    e1.reset()
-    e2.reset()
-    gen = torch.Generator(device="cuda").manual_seed(5)
-    for t in range(12):
-        a = torch.rand((B, N, 2), generator=gen, device="cuda") * 20 - 10
-        e1.step(a)
-        e2.step(a)
-        assert torch.equal(e1.obs, e2.obs) and torch.equal(e1.reward, e2.reward) and torch.equal(e1.done, e2.done)
-        assert torch.equal(e1.reset_mask, e2.reset_mask)
-    assert torch.equal(e1.state.blob, e2.state.blob)
 
 
 @pytest.mark.parametrize("n", [11, 17, 20, 24, 25])

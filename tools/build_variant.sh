@@ -1,6 +1,6 @@
 #!/bin/bash
 # Build a kernel variant of libuavca.so with extra -D flags (A/B experiments; load it with UAVCA_LIB=<path>).
-#   tools/build_variant.sh NAME [-DUAVCA_TMA_MINB=5 ...]  ->  build/variants/libuavca_NAME.so
+#   tools/build_variant.sh NAME [-DUAVCA_ROLLOUT_MINB=6 ...]  ->  build/variants/libuavca_NAME.so
 set -e
 name=$1; shift
 root=$(cd "$(dirname "$0")/.." && pwd)

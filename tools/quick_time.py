@@ -1,5 +1,5 @@
 """Device time per step of one workload (CUDA-graph replay over a ring of batches larger than L2), no CPU legs.
-    python tools/quick_time.py [N] [B] [steps]      (UAVCA_LIB / UAVCA_STEP_PATH select the kernel variant)"""
+    python tools/quick_time.py [N] [B] [steps]      (UAVCA_LIB selects the library variant)"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -51,5 +51,5 @@ for _ in range(3):
     st.synchronize()
     best = min(best, e0.elapsed_time(e1) * 1e3 / (reps * G_STEPS))
 alg = 107 + 24 / N
-print(f"{os.environ.get('UAVCA_LIB', 'default').split('/')[-1]:28s} path={os.environ.get('UAVCA_STEP_PATH', 'lanes'):5s} streams={S} N={N} B={B} ring={ring} "
+print(f"{os.environ.get('UAVCA_LIB', 'default').split('/')[-1]:28s} streams={S} N={N} B={B} ring={ring} "
       f"{best:9.2f} us/step  {B * N / best / 1e3:7.2f} G UAV-steps/s  frac {B * N * alg / best / 1e3 / 6515.7:.3f}", flush=True)
