@@ -14,6 +14,7 @@ import numpy as np
 import torch
 
 from . import _capi, ops
+from .replay import PrioritizedDeviceReplay
 from ._capi import (ACTION_CARTESIAN, ACTION_POLAR, ACTION_SCALED, KIND_MULTI, KIND_SINGLE, RESET_ON_ALL_DONE,  # noqa: F401
                     RESET_ON_ANY_DONE, RESET_ON_DONE0, SOURCE_PHILOX, SOURCE_POOL)
 
@@ -448,7 +449,8 @@ class BatchedMultiUAVWorld2D(_BatchedBase):
         """`step(action)` that also appends every UAV's transition (prev_obs, action, reward, next observation before any
         auto-reset, 1 - done) to `replay` (a `DeviceReplay`) in the SAME launch — env.step followed by the N
         `memory.push` calls of a training step (test_sac_multi.py:99-103).  `prev_obs` is the observation the action was
-        taken on; it must not be the tensor this step writes (`env.obs`): ping-pong two buffers with `set_obs_buffer`."""
+        taken on; it must not be the tensor this step writes (`env.obs`): ping-pong two buffers with `set_obs_buffer`.
+        A `PrioritizedDeviceReplay` is synced after the launch (one more launch): the new slots take its largest priority."""
         action = self._check_action(action)
         if prev_obs.data_ptr() == self.obs.data_ptr():
             raise ValueError("prev_obs is the buffer this step writes its observation into (use set_obs_buffer)")
@@ -470,6 +472,8 @@ class BatchedMultiUAVWorld2D(_BatchedBase):
             ops.step_multi_replay(self._h, self.state.blob, action, _ACTION_MODES[action_mode], bool(evaluate), prev_obs,
                                   self.obs, self.reward, self.done, self.final_obs, self.reset_mask, replay.state,
                                   replay.action, replay.reward, replay.next_state, replay.mask, replay.meta)
+        if isinstance(replay, PrioritizedDeviceReplay):
+            replay.sync()
         info = {"distance": 0, "reset_mask": self.reset_mask}
         if self.final_obs is not None:
             info["final_obs"] = self.final_obs

@@ -773,6 +773,81 @@ int uavca_replay_sample(const float* ring_obs, const float* ring_action, const f
   return 0;
 }
 
+// Prioritized replay: the tree of a ring of `capacity` slots has L leaves, the least power of two >= capacity.
+static int per_check_tree(const char* what, const double* tree, int64_t L, int64_t capacity, const int64_t* per_meta) {
+  if (!tree || !per_meta) return fail(-1, "null argument");
+  if (capacity <= 0 || capacity > UAVCA_PER_MAX_CAPACITY)
+    return fail(-1, std::string(what) + ": capacity " + std::to_string(capacity) + " is outside 1..2^26");
+  int64_t want = 1;
+  while (want < capacity) want <<= 1;
+  if (L != want)
+    return fail(-1, std::string(what) + ": L = " + std::to_string(L) + ", but a ring of " + std::to_string(capacity) +
+                        " slots needs L = " + std::to_string(want));
+  if (misaligned(tree, 8) || misaligned(per_meta, 8)) return fail(-1, "misaligned buffer: tree and per_meta need 8-byte alignment");
+  return 0;
+}
+
+static int per_device(const char* what, const void* p) {
+  cudaPointerAttributes at{};
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess || at.type != cudaMemoryTypeDevice) {
+    cudaGetLastError();
+    return fail(-1, std::string(what) + ": tree is not a device pointer");
+  }
+  return at.device;
+}
+
+int uavca_per_sync(double* tree, int64_t L, int64_t* per_meta, const int64_t* ring_meta, int64_t capacity, void* stream) {
+  if (int rc = per_check_tree("uavca_per_sync", tree, L, capacity, per_meta)) return rc;
+  if (!ring_meta) return fail(-1, "null argument");
+  const int dev = per_device("uavca_per_sync", tree);
+  if (dev < 0) return -1;
+  DeviceGuard g(dev);
+  cudaError_t e = launch_per_sync(tree, L, reinterpret_cast<long long*>(per_meta), reinterpret_cast<const long long*>(ring_meta),
+                                  capacity, (cudaStream_t)stream);
+  if (e != cudaSuccess) return fail_cuda("uavca_per_sync", e);
+  return 0;
+}
+
+int uavca_per_update(double* tree, int64_t L, int64_t capacity, int64_t* per_meta, const int64_t* index, const double* priority,
+                     int64_t n, void* stream) {
+  if (int rc = per_check_tree("uavca_per_update", tree, L, capacity, per_meta)) return rc;
+  if (n < 0 || n > capacity) return fail(-1, "uavca_per_update: n must be in 0..capacity");
+  if (n == 0) return 0;
+  if (!index || !priority) return fail(-1, "null argument");
+  if (misaligned(index, 8) || misaligned(priority, 8)) return fail(-1, "misaligned buffer: index and priority need 8-byte alignment");
+  const int dev = per_device("uavca_per_update", tree);
+  if (dev < 0) return -1;
+  DeviceGuard g(dev);
+  cudaError_t e = launch_per_update(tree, L, capacity, reinterpret_cast<long long*>(per_meta),
+                                    reinterpret_cast<const long long*>(index), priority, n, (cudaStream_t)stream);
+  if (e != cudaSuccess) return fail_cuda("uavca_per_update", e);
+  return 0;
+}
+
+int uavca_per_sample(const float* ring_obs, const float* ring_action, const float* ring_reward, const float* ring_next_obs,
+                     const float* ring_mask, int64_t capacity, int32_t obs_dim, int32_t act_dim, const int64_t* ring_meta,
+                     double* tree, int64_t L, int64_t batch, double beta, uint64_t seed, uint64_t draw, float* out_obs,
+                     float* out_action, float* out_reward, float* out_next_obs, float* out_mask, int64_t* out_index,
+                     float* out_weight, void* stream) {
+  if (!ring_obs || !ring_action || !ring_reward || !ring_next_obs || !ring_mask || !ring_meta || !out_obs || !out_action ||
+      !out_reward || !out_next_obs || !out_mask || !out_index || !out_weight)
+    return fail(-1, "null argument");
+  if (!tree) return fail(-1, "null argument");
+  if (int rc = per_check_tree("uavca_per_sample", tree, L, capacity, ring_meta)) return rc;
+  if (batch < 0 || batch >= ((int64_t)1 << 26) || obs_dim <= 0 || act_dim <= 0) return fail(-1, "bad sizes");
+  if (!std::isfinite(beta)) return fail(-1, "uavca_per_sample: beta must be finite");
+  if (misaligned(out_index, 8)) return fail(-1, "misaligned buffer: out_index needs 8-byte alignment");
+  const int dev = per_device("uavca_per_sample", tree);
+  if (dev < 0) return -1;
+  DeviceGuard g(dev);
+  cudaError_t e = launch_per_sample(ring_obs, ring_action, ring_reward, ring_next_obs, ring_mask, obs_dim, act_dim,
+                                    reinterpret_cast<const long long*>(ring_meta), tree, L, batch, beta, seed, draw, out_obs,
+                                    out_action, out_reward, out_next_obs, out_mask, reinterpret_cast<long long*>(out_index),
+                                    out_weight, (cudaStream_t)stream);
+  if (e != cudaSuccess) return fail_cuda("uavca_per_sample", e);
+  return 0;
+}
+
 int uavca_step_multi_replay(uavca_handle* h, void* state, const float* action, int action_mode, int evaluate,
                             const float* prev_obs, float* obs, float* reward, uint8_t* done, float* final_obs,
                             uint8_t* reset_mask, float* ring_obs, float* ring_action, float* ring_reward, float* ring_next_obs,

@@ -32,7 +32,9 @@ constexpr unsigned kMaxResetAttempts = 4096u;  // the reference would loop forev
 //   actions  (env, t >> 1, 3 << 16 | uav, t >> 33)                uav < 2^16
 //   policy   (row, ctr, 4 << 16 | row >> 32, ctr >> 32)          row < 2^48     (uavca_policy.cu)
 //   sampler  (sample, ctr, 5 << 16 | sample >> 32, ctr >> 32)    sample < 2^48  (replay_sample_kernel)
-enum : int { kStreamPos = 0, kStreamTgt = 1, kStreamVel = 2, kStreamAct = 3, kStreamPolicy = 4, kStreamSample = 5 };
+//   per      (sample, ctr, 6 << 16 | sample >> 32, ctr >> 32)    sample < 2^48  (per_sample_kernel, uavca_per.cu)
+enum : int { kStreamPos = 0, kStreamTgt = 1, kStreamVel = 2, kStreamAct = 3, kStreamPolicy = 4, kStreamSample = 5,
+             kStreamPerSample = 6 };
 
 // Constants derived once on the host from uavca_config (capi.cu: derive_consts).
 struct Consts {

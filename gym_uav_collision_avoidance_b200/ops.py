@@ -155,6 +155,59 @@ def replay_sample(ring_obs: torch.Tensor, ring_action: torch.Tensor, ring_reward
                                                  _ptr(out_index), _stream(ring_obs)), "uavca_replay_sample")
 
 
+def _per_tree(tree: torch.Tensor, per_meta: Optional[torch.Tensor]) -> int:
+    """Checks the sum-tree and per_meta tensors of prioritized replay; returns L."""
+    if tree.dtype != torch.float64 or tree.dim() != 1 or tree.numel() < 2 or tree.numel() % 2:
+        raise _capi.UavcaError("the priority tree is a 1-D float64 tensor of 2L elements")
+    if per_meta is not None and (per_meta.dtype != torch.int64 or per_meta.numel() != 5):
+        raise _capi.UavcaError("per_meta is an int64 tensor of 5 elements")
+    return tree.numel() // 2
+
+
+@torch.library.custom_op("uavca::per_sync", mutates_args=("tree", "per_meta"))
+def per_sync(tree: torch.Tensor, per_meta: torch.Tensor, ring_meta: torch.Tensor, capacity: int) -> None:
+    """Give the slots appended since the last sync the largest priority so far (one launch, no host sync)."""
+    _need_cuda(tree, per_meta, ring_meta)
+    L = _per_tree(tree, per_meta)
+    _capi.check(_capi.load().uavca_per_sync(tree.data_ptr(), L, per_meta.data_ptr(), ring_meta.data_ptr(), capacity,
+                                            _stream(tree)), "uavca_per_sync")
+
+
+@torch.library.custom_op("uavca::per_update", mutates_args=("tree", "per_meta"))
+def per_update(tree: torch.Tensor, per_meta: torch.Tensor, index: torch.Tensor, priority: torch.Tensor, capacity: int) -> None:
+    """Set leaf index[j] to priority[j] (last occurrence wins) and form the ancestors again; an update with a bad index or
+    priority is dropped whole on the device and counted in per_meta[4]."""
+    _need_cuda(tree, per_meta, index, priority)
+    L = _per_tree(tree, per_meta)
+    if index.dtype != torch.int64 or priority.dtype != torch.float64 or index.numel() != priority.numel():
+        raise _capi.UavcaError("per_update takes int64 indices and as many float64 priorities")
+    _capi.check(_capi.load().uavca_per_update(tree.data_ptr(), L, capacity, per_meta.data_ptr(), index.data_ptr(),
+                                              priority.data_ptr(), index.numel(), _stream(tree)), "uavca_per_update")
+
+
+@torch.library.custom_op("uavca::per_sample", mutates_args=("tree", "out_obs", "out_action", "out_reward", "out_next_obs",
+                                                           "out_mask", "out_index", "out_weight"))
+def per_sample(ring_obs: torch.Tensor, ring_action: torch.Tensor, ring_reward: torch.Tensor, ring_next_obs: torch.Tensor,
+               ring_mask: torch.Tensor, ring_meta: torch.Tensor, tree: torch.Tensor, batch: int, beta: float, seed: int,
+               draw: int, out_obs: torch.Tensor, out_action: torch.Tensor, out_reward: torch.Tensor, out_next_obs: torch.Tensor,
+               out_mask: torch.Tensor, out_index: torch.Tensor, out_weight: torch.Tensor) -> None:
+    """Stratified proportional draw of `batch` slots from the sum-tree, gathered with importance weights, in one launch.
+    (`tree` is listed as mutated: its element 0 is the launch's CTA ticket.)"""
+    _need_cuda(ring_obs, ring_action, ring_reward, ring_next_obs, ring_mask, ring_meta, tree, out_obs, out_action,
+               out_reward, out_next_obs, out_mask, out_index, out_weight)
+    L = _per_tree(tree, None)
+    if out_index.dtype != torch.int64 or out_weight.dtype != torch.float32 or out_index.numel() != batch or \
+            out_weight.numel() != batch or out_reward.numel() != batch:
+        raise _capi.UavcaError("per_sample: out_index int64 [batch], out_weight float32 [batch]")
+    cap = ring_reward.numel()
+    _capi.check(_capi.load().uavca_per_sample(ring_obs.data_ptr(), ring_action.data_ptr(), ring_reward.data_ptr(),
+                                              ring_next_obs.data_ptr(), ring_mask.data_ptr(), cap, ring_obs.numel() // cap,
+                                              ring_action.numel() // cap, ring_meta.data_ptr(), tree.data_ptr(), L, batch,
+                                              float(beta), seed, draw, out_obs.data_ptr(), out_action.data_ptr(),
+                                              out_reward.data_ptr(), out_next_obs.data_ptr(), out_mask.data_ptr(),
+                                              out_index.data_ptr(), out_weight.data_ptr(), _stream(tree)), "uavca_per_sample")
+
+
 @torch.library.custom_op("uavca::step_multi_replay",
                          mutates_args=("state", "obs", "reward", "done", "final_obs", "reset_mask", "ring_obs", "ring_action",
                                        "ring_reward", "ring_next_obs", "ring_mask", "ring_meta"))

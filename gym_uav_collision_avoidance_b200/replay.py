@@ -96,3 +96,86 @@ class DeviceReplay:
         else:
             idx = torch.randint(0, size, (batch_size,), generator=self.gen, device=self.device)
         return self.state[idx], self.action[idx], self.reward[idx], self.next_state[idx], self.mask[idx]
+
+
+PER_MAX_CAPACITY = 1 << 26  # UAVCA_PER_MAX_CAPACITY (include/uavca.h)
+
+
+class PrioritizedDeviceReplay(DeviceReplay):
+    """`DeviceReplay` with proportional prioritized sampling (Schaul et al. 2016, as the Ape-X learner uses it, Horgan et
+    al. 2018): a float64 sum-tree over the ring's slots lives on the device next to the ring (`tree`, `per_meta`; layout in
+    include/uavca.h).  New transitions enter with the largest priority set so far (1.0 at first); the learner draws
+    stratified batches with importance weights and writes back (|td| + eps)^alpha.  Every call is one launch with no host
+    synchronisation, so both the acting step and the learner step can be captured in CUDA graphs.  The inherited `sample` /
+    `sample_fused` keep drawing uniformly or by recency.
+
+    Keep the tree in step with the ring: `push` syncs after its append, and `BatchedMultiUAVWorld2D.step_replay` syncs after
+    its fused append.  An append that reaches the ring another way must be followed by `sync()` before the next append;
+    otherwise the sync cannot tell which slots are new, gives every filled slot the largest priority and counts the miss
+    in `missed_syncs`."""
+
+    def __init__(self, capacity: int, obs_dim: int, act_dim: int = 2, device="cuda", seed: Optional[int] = None,
+                 alpha: float = 0.6, eps: float = 1e-6):
+        if not 1 <= int(capacity) <= PER_MAX_CAPACITY:
+            raise ValueError(f"a prioritized ring holds 1 to 2^26 slots, not {capacity}")
+        super().__init__(capacity, obs_dim, act_dim, device, seed)
+        self.alpha, self.eps = float(alpha), float(eps)
+        self.leaves = 1 << (self.capacity - 1).bit_length()
+        self.tree = torch.zeros(2 * self.leaves, dtype=torch.float64, device=self.device)
+        # [0] appends and [1] head at the last sync, [2] largest priority so far (float64 bits), [3] missed syncs,
+        # [4] refused updates
+        self.per_meta = torch.zeros(5, dtype=torch.int64, device=self.device)
+        self.per_meta[2:3].view(torch.float64).fill_(1.0)
+        self._per_draws = 0
+
+    def push(self, state: torch.Tensor, action: torch.Tensor, reward: torch.Tensor, next_state: torch.Tensor,
+             done: torch.Tensor) -> None:
+        """`DeviceReplay.push`, then `sync()`: the new transitions take the largest priority so far.  Two launches."""
+        super().push(state, action, reward, next_state, done)
+        self.sync()
+
+    def sync(self) -> None:
+        """Give every slot appended since the last sync the largest priority so far (one launch, no host sync)."""
+        ops.per_sync(self.tree, self.per_meta, self.meta, self.capacity)
+
+    def sample_prioritized(self, batch_size: int, beta: float, out=None):
+        """Draw `batch_size` transitions with probability leaf / total, stratified over `batch_size` equal strata of the
+        total, in ONE launch: -> (state, action, reward, next_state, mask, index int64, weight float32).  weight =
+        (size * P)^-beta divided by the batch's largest.  `out` reuses a previous result's tensors.  `beta` is frozen into
+        a captured CUDA graph; the draws of a captured learner step change as appends advance the ring (as `sample_fused`).
+        An empty ring yields slot 0 with weight 0."""
+        if out is None:
+            kw = dict(dtype=torch.float32, device=self.device)
+            out = (torch.empty((batch_size, self.obs_dim), **kw), torch.empty((batch_size, self.act_dim), **kw),
+                   torch.empty(batch_size, **kw), torch.empty((batch_size, self.obs_dim), **kw), torch.empty(batch_size, **kw),
+                   torch.empty(batch_size, dtype=torch.int64, device=self.device), torch.empty(batch_size, **kw))
+        ops.per_sample(self.state, self.action, self.reward, self.next_state, self.mask, self.meta, self.tree, batch_size,
+                       float(beta), self._sample_seed, self._per_draws, *out)
+        self._per_draws += 1
+        return out
+
+    def update_priorities(self, index: torch.Tensor, td_error: torch.Tensor) -> None:
+        """Set the priorities of slots `index` to (|td_error| + eps)^alpha, formed in float64 by torch; the last occurrence
+        of a repeated slot wins.  An out-of-range index or a NaN / infinite error drops the whole update on the device
+        (counted in `refused_updates`).  One launch beside torch's element-wise ops, no host sync."""
+        index = index.reshape(-1)
+        td = td_error.reshape(-1)
+        if index.numel() != td.numel():
+            raise ValueError(f"{index.numel()} slots but {td.numel()} TD errors")
+        p = (td.detach().to(torch.float64).abs() + self.eps).pow(self.alpha)
+        ops.per_update(self.tree, self.per_meta, index.to(torch.int64).contiguous(), p.contiguous(), self.capacity)
+
+    @property
+    def max_priority(self) -> float:
+        """The largest priority set so far (synchronises with the device)."""
+        return float(self.per_meta[2:3].view(torch.float64).item())
+
+    @property
+    def missed_syncs(self) -> int:
+        """Syncs that found more than one append since the previous one (synchronises with the device)."""
+        return int(self.per_meta[3].item())
+
+    @property
+    def refused_updates(self) -> int:
+        """Priority updates dropped for an out-of-range slot or a negative / non-finite priority (synchronises)."""
+        return int(self.per_meta[4].item())

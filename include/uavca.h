@@ -15,6 +15,8 @@
  *   uavca_rollout      <- the random-action driver loops    run.py:10-16, run_multi.py:10-16 (K x env.step per call)
  *   uavca_step_multi_replay <- env.step + the N memory.push calls of a training step   test_sac_multi.py:99-103
  *   uavca_replay_push(_dev) / uavca_replay_sample <- ReplayMemory.push / .sample   pytorch_sac_temp/replay_memory.py:15-24
+ *   uavca_per_sync / uavca_per_update / uavca_per_sample <- no reference counterpart: prioritized replay over the device ring
+ *                         (Schaul et al. 2016, the sum-tree of the Ape-X learner, Horgan et al. 2018)
  *   uavca_stats        <- env.steps / target_reach_count / collision_count  multi_uav_world_2d.py:166-168,209,221,238
  *   uavca_config       <- constructor kwargs              multi_uav_world_2d.py:13-28, uav_world_2d.py:14-26
  *
@@ -35,7 +37,7 @@
 extern "C" {
 #endif
 
-#define UAVCA_VERSION 203
+#define UAVCA_VERSION 204
 
 /* world kinds */
 #define UAVCA_KIND_MULTI 0  /* MultiUAVWorld2D: N UAVs per env, 10-feature observation */
@@ -244,6 +246,56 @@ int uavca_replay_sample(const float* ring_obs, const float* ring_action, const f
                         const float* ring_mask, int64_t capacity, int32_t obs_dim, int32_t act_dim, const int64_t* ring_meta,
                         int64_t batch, uint64_t seed, uint64_t draw, int recency_weighted, float* out_obs, float* out_action,
                         float* out_reward, float* out_next_obs, float* out_mask, int64_t* out_index, void* stream);
+
+/* Prioritized replay over the device ring (Schaul et al. 2016): a sum-tree over the ring's slots, owned by the caller like
+ * the ring and kept in step with it through the ring's device-side head, so that every call is asynchronous and can be
+ * captured in a CUDA graph.  No existing call reads or writes it.
+ *   tree     double [2L], L = the least power of two >= capacity; zero-initialised.  The leaf of slot s is tree[L + s];
+ *            internal node k (1 <= k < L) holds exactly tree[2k] + tree[2k+1] (one IEEE float64 addition, left child first),
+ *            so the tree is a pure function of its leaves; tree[1] is the total.  Leaves of slots never written are 0.
+ *            tree[0] is no node: the multi-CTA calls keep their CTA ticket there (0 between calls), so the calls on one
+ *            tree must be ordered (one stream, or events).
+ *   per_meta int64 [5]: [0] ring_meta[3] at the last sync, [1] ring_meta[0] at the last sync, [2] the largest priority set
+ *            so far as float64 bits (initialise it to 1.0), [3] syncs that found more than one append, [4] refused updates;
+ *            zero-initialise the rest.
+ * capacity <= UAVCA_PER_MAX_CAPACITY; every call checks capacity and L (and its other sizes) before it launches. */
+#define UAVCA_PER_MAX_CAPACITY ((int64_t)1 << 26)
+
+/* Give every slot appended since the last sync the priority per_meta[2], then form their ancestors again; one launch.
+ * With d = ring_meta[3] - per_meta[0]:
+ *   d == 0  nothing changes;
+ *   d == 1  the new slots are the n slots from per_meta[1] on, wrapping at capacity, n = (ring_meta[0] - per_meta[1]) mod
+ *           capacity.  n == 0 is a full-capacity append: an append of M = 0 transitions launches nothing and leaves
+ *           ring_meta[3] as it is (uavca_replay_push_dev; uavca_step_multi_replay always appends B * N >= 1), so it can
+ *           never be mistaken for one;
+ *   d >  1  which slots are new can no longer be told: every filled slot (0 .. ring_meta[2] - 1) takes per_meta[2] and
+ *           per_meta[3] counts the miss.  Sync after every append to keep the learner's priorities.
+ * Then per_meta[0..1] = ring_meta[3], ring_meta[0]. */
+int uavca_per_sync(double* tree, int64_t L, int64_t* per_meta, const int64_t* ring_meta, int64_t capacity, void* stream);
+
+/* Set leaf index[j] to priority[j] for j < n (index int64 [n], priority double [n], n <= capacity), raise per_meta[2] to the
+ * largest of them and form their ancestors again; one launch, one CTA (sized for learner batches of a few hundred slots).
+ * The caller forms priority = (|td| + eps)^alpha itself (in float64), so the tree does not depend on the device's pow.
+ * Repeated slots: the last occurrence wins, as a sequential loop would leave it.  An index outside 0..capacity-1 or a
+ * priority that is negative or not finite is found on the device; reporting it would need a host synchronisation, so the
+ * whole update is dropped instead: tree and per_meta[2] stay as they are and per_meta[4] counts it. */
+int uavca_per_update(double* tree, int64_t L, int64_t capacity, int64_t* per_meta, const int64_t* index, const double* priority,
+                     int64_t n, void* stream);
+
+/* Draw `batch` slots in proportion to their leaves and gather them as uavca_replay_sample does, in ONE launch; out_index
+ * int64 [batch] receives the slots and out_weight float [batch] the importance weights.  Stratified: sample j takes
+ * u = (j + U) / batch * tree[1] in float64, U the 53-bit uniform of words 0 and 1 (u53) of the Philox4x32-10 block with key
+ * seed and counter (j, ctr, 6 << 16 | j >> 32, ctr >> 32), ctr = draw + ring_meta[3].  From node 1 it goes left when
+ * u < tree[2k] or tree[2k+1] == 0, else u -= tree[2k] and right; the leaf reached is the slot (never an empty one while
+ * the total is nonzero).  Weight w = (size * leaf / tree[1])^-beta, size = ring_meta[2], divided by the largest w of the
+ * batch.  An empty tree (tree[1] == 0) yields slot 0 with weight 0.  beta is a host argument: a captured graph replays
+ * the beta it was captured with.  Like uavca_replay_sample, a captured learner step draws afresh as appends advance
+ * ring_meta[3]. */
+int uavca_per_sample(const float* ring_obs, const float* ring_action, const float* ring_reward, const float* ring_next_obs,
+                     const float* ring_mask, int64_t capacity, int32_t obs_dim, int32_t act_dim, const int64_t* ring_meta,
+                     double* tree, int64_t L, int64_t batch, double beta, uint64_t seed, uint64_t draw, float* out_obs,
+                     float* out_action, float* out_reward, float* out_next_obs, float* out_mask, int64_t* out_index,
+                     float* out_weight, void* stream);
 
 /* uavca_step_multi with the replay append folded into the SAME launch ("next" row; MultiUAVWorld2D.step followed by the N
  * memory.push calls of test_sac_multi.py:99-103).  Besides everything uavca_step_multi writes, UAV m's transition goes to
