@@ -9,7 +9,8 @@ Reference, per env step (one env, N agents):            Here, per env step (B en
   every 10 episodes: 10 evaluation episodes, SR / CR       evaluation batch with RESET_ON_ALL_DONE, evaluate=True
 
 The learner (SAC.update_parameters, pytorch_sac_temp/sac.py:46-98) is stock PyTorch and out of scope; `replay.sample(256)`
-/ `replay.sample_fused(256)` (one launch, slots drawn on the device) return exactly the five tensors it consumes.
+/ `replay.sample_fused(256)` (one launch, slots drawn on the device) return exactly the five tensors it consumes;
+`replay.sample_nstep(256, n, gamma, stride)` returns n-step returns for the same learner.
 
     python examples/rollout_sac_multi.py [--envs 16384] [--agents 10] [--steps 2000]
 """
@@ -52,6 +53,10 @@ def main(argv=None):
     print(f"collected {args.steps * args.envs * args.agents:,} transitions in {dt:.2f} s "
           f"({args.steps * args.envs / dt:,.0f} env-steps/s, eager launches); replay holds {len(replay):,}; "
           f"sampled batch shapes {[tuple(t.shape) for t in batch]}")
+    # 3-step returns for the same learner: successors are envs * agents slots apart
+    nstep = replay.sample_nstep(256, n=3, gamma=0.99, stride=args.envs * args.agents)
+    print(f"3-step batch shapes {[tuple(t.shape) for t in nstep]} (state, action, reward_3, next_state_3, discount); "
+          f"mean discount {nstep[4].mean().item():.3f}")
 
     # evaluation protocol (:136-179): evaluate=True (out-of-bounds does not end the episode), stop at all(dones)
     ev = G.BatchedMultiUAVWorld2D(args.eval_envs, num_agents=args.agents, reset_mode=G.RESET_ON_ALL_DONE,

@@ -82,6 +82,9 @@ SYMBOLS = {
                                            _VP, C.c_int64, _VP, _VP]),
     "uavca_replay_sample": (C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int64, C.c_int32, C.c_int32, _VP, C.c_int64, C.c_uint64,
                                       C.c_uint64, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "uavca_replay_sample_nstep": (C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int64, C.c_int32, C.c_int32, _VP, C.c_int64,
+                                            C.c_uint64, C.c_uint64, C.c_int, C.c_int64, C.c_int32, C.c_double, _VP, _VP, _VP,
+                                            _VP, _VP, _VP, _VP]),
     "uavca_replay_push_dev": (C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int64, C.c_int32, C.c_int32, _VP, _VP, _VP, _VP, _VP,
                                         C.c_int64, _VP, _VP]),
     "uavca_replay_push": (C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int64, C.c_int32, C.c_int32, _VP, _VP, _VP, _VP, _VP,
@@ -90,6 +93,9 @@ SYMBOLS = {
     "uavca_per_update": (C.c_int, [_VP, C.c_int64, C.c_int64, _VP, _VP, _VP, C.c_int64, _VP]),
     "uavca_per_sample": (C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int64, C.c_int32, C.c_int32, _VP, _VP, C.c_int64, C.c_int64,
                                    C.c_double, C.c_uint64, C.c_uint64, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "uavca_per_sample_nstep": (C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int64, C.c_int32, C.c_int32, _VP, _VP, C.c_int64,
+                                         C.c_int64, C.c_double, C.c_int64, C.c_int32, C.c_double, C.c_uint64, C.c_uint64,
+                                         _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     "uavca_policy_act": (C.c_int, [_VP, C.c_int64, _VP, _VP, _VP, _VP, _VP, _VP, C.c_uint64, C.c_uint64, _VP, _VP, _VP, _VP]),
     "uavca_launch_count": (C.c_int64, [_VP]),
 }

@@ -9,7 +9,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(_HERE, "libuavca.so")
 SOURCES = ["uavca_kernels.cu", "uavca_policy.cu", "uavca_per.cu", "uavca_capi.cu"]
-HEADERS = ["uavca_device.cuh", "uavca_multi.cuh", "uavca_seq.cuh", "uavca_cta.cuh", "uavca_host.h",
+HEADERS = ["uavca_device.cuh", "uavca_multi.cuh", "uavca_seq.cuh", "uavca_cta.cuh", "uavca_nstep.cuh", "uavca_host.h",
            os.path.join("..", "..", "include", "uavca.h")]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-Xcompiler", "-fPIC"]
 

@@ -773,6 +773,43 @@ int uavca_replay_sample(const float* ring_obs, const float* ring_action, const f
   return 0;
 }
 
+// n-step arguments, checked before any launch: 1 <= n <= 16 (one lane of the sample's 16 per link), 1 <= stride <=
+// capacity, gamma finite in [0, 1]
+static int nstep_check(const char* what, int64_t capacity, int64_t stride, int32_t n, double gamma) {
+  if (n < 1 || n > 16) return fail(-1, std::string(what) + ": n = " + std::to_string(n) + " is outside 1..16");
+  if (stride < 1 || stride > capacity)
+    return fail(-1, std::string(what) + ": stride = " + std::to_string(stride) + " is outside 1..capacity (" +
+                        std::to_string(capacity) + ")");
+  if (!(gamma >= 0.0 && gamma <= 1.0)) return fail(-1, std::string(what) + ": gamma must be finite and in [0, 1]");
+  return 0;
+}
+
+int uavca_replay_sample_nstep(const float* ring_obs, const float* ring_action, const float* ring_reward,
+                              const float* ring_next_obs, const float* ring_mask, int64_t capacity, int32_t obs_dim,
+                              int32_t act_dim, const int64_t* ring_meta, int64_t batch, uint64_t seed, uint64_t draw,
+                              int recency_weighted, int64_t stride, int32_t n, double gamma, float* out_obs,
+                              float* out_action, float* out_reward, float* out_next_obs, float* out_discount,
+                              int64_t* out_index, void* stream) {
+  if (!ring_obs || !ring_action || !ring_reward || !ring_next_obs || !ring_mask || !ring_meta || !out_obs || !out_action ||
+      !out_reward || !out_next_obs || !out_discount)
+    return fail(-1, "null argument");
+  if (batch < 0 || obs_dim <= 0 || act_dim <= 0 || capacity <= 0 || capacity >= ((int64_t)1 << 32)) return fail(-1, "bad sizes");
+  if (int rc = nstep_check("uavca_replay_sample_nstep", capacity, stride, n, gamma)) return rc;
+  cudaPointerAttributes at{};
+  if (cudaPointerGetAttributes(&at, ring_obs) != cudaSuccess || at.type != cudaMemoryTypeDevice) {
+    cudaGetLastError();
+    return fail(-1, "uavca_replay_sample_nstep: ring_obs is not a device pointer");
+  }
+  DeviceGuard g(at.device);
+  cudaError_t e = launch_replay_sample_nstep(ring_obs, ring_action, ring_reward, ring_next_obs, ring_mask, capacity, obs_dim,
+                                             act_dim, reinterpret_cast<const long long*>(ring_meta), batch, seed, draw,
+                                             recency_weighted, stride, n, gamma, out_obs, out_action, out_reward,
+                                             out_next_obs, out_discount, reinterpret_cast<long long*>(out_index),
+                                             (cudaStream_t)stream);
+  if (e != cudaSuccess) return fail_cuda("uavca_replay_sample_nstep", e);
+  return 0;
+}
+
 // Prioritized replay: the tree of a ring of `capacity` slots has L leaves, the least power of two >= capacity.
 static int per_check_tree(const char* what, const double* tree, int64_t L, int64_t capacity, const int64_t* per_meta) {
   if (!tree || !per_meta) return fail(-1, "null argument");
@@ -845,6 +882,32 @@ int uavca_per_sample(const float* ring_obs, const float* ring_action, const floa
                                     out_action, out_reward, out_next_obs, out_mask, reinterpret_cast<long long*>(out_index),
                                     out_weight, (cudaStream_t)stream);
   if (e != cudaSuccess) return fail_cuda("uavca_per_sample", e);
+  return 0;
+}
+
+int uavca_per_sample_nstep(const float* ring_obs, const float* ring_action, const float* ring_reward,
+                           const float* ring_next_obs, const float* ring_mask, int64_t capacity, int32_t obs_dim,
+                           int32_t act_dim, const int64_t* ring_meta, double* tree, int64_t L, int64_t batch, double beta,
+                           int64_t stride, int32_t n, double gamma, uint64_t seed, uint64_t draw, float* out_obs,
+                           float* out_action, float* out_reward, float* out_next_obs, float* out_discount,
+                           int64_t* out_index, float* out_weight, void* stream) {
+  if (!ring_obs || !ring_action || !ring_reward || !ring_next_obs || !ring_mask || !ring_meta || !out_obs || !out_action ||
+      !out_reward || !out_next_obs || !out_discount || !out_index || !out_weight)
+    return fail(-1, "null argument");
+  if (!tree) return fail(-1, "null argument");
+  if (int rc = per_check_tree("uavca_per_sample_nstep", tree, L, capacity, ring_meta)) return rc;
+  if (batch < 0 || batch >= ((int64_t)1 << 26) || obs_dim <= 0 || act_dim <= 0) return fail(-1, "bad sizes");
+  if (!std::isfinite(beta)) return fail(-1, "uavca_per_sample_nstep: beta must be finite");
+  if (int rc = nstep_check("uavca_per_sample_nstep", capacity, stride, n, gamma)) return rc;
+  if (misaligned(out_index, 8)) return fail(-1, "misaligned buffer: out_index needs 8-byte alignment");
+  const int dev = per_device("uavca_per_sample_nstep", tree);
+  if (dev < 0) return -1;
+  DeviceGuard g(dev);
+  cudaError_t e = launch_per_sample_nstep(ring_obs, ring_action, ring_reward, ring_next_obs, ring_mask, capacity, obs_dim,
+                                          act_dim, reinterpret_cast<const long long*>(ring_meta), tree, L, batch, beta, stride,
+                                          n, gamma, seed, draw, out_obs, out_action, out_reward, out_next_obs, out_discount,
+                                          reinterpret_cast<long long*>(out_index), out_weight, (cudaStream_t)stream);
+  if (e != cudaSuccess) return fail_cuda("uavca_per_sample_nstep", e);
   return 0;
 }
 

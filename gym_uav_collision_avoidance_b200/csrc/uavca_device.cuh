@@ -33,6 +33,8 @@ constexpr unsigned kMaxResetAttempts = 4096u;  // the reference would loop forev
 //   policy   (row, ctr, 4 << 16 | row >> 32, ctr >> 32)          row < 2^48     (uavca_policy.cu)
 //   sampler  (sample, ctr, 5 << 16 | sample >> 32, ctr >> 32)    sample < 2^48  (replay_sample_kernel)
 //   per      (sample, ctr, 6 << 16 | sample >> 32, ctr >> 32)    sample < 2^48  (per_sample_kernel, uavca_per.cu)
+// The n-step samplers (replay_sample_nstep_kernel, per_sample_kernel<true>) draw on the streams 5 and 6 of their one-step
+// siblings through the same draw code, so the same (seed, draw, appends) gives the same slots: no stream of their own.
 enum : int { kStreamPos = 0, kStreamTgt = 1, kStreamVel = 2, kStreamAct = 3, kStreamPolicy = 4, kStreamSample = 5,
              kStreamPerSample = 6 };
 

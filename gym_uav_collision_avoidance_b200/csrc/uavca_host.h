@@ -31,6 +31,12 @@ cudaError_t launch_replay_sample(const float* r_obs, const float* r_act, const f
                                  const float* r_mask, long long capacity, int obs_dim, int act_dim, const long long* meta,
                                  long long batch, unsigned long long seed, unsigned long long draw, int recency, float* o_obs,
                                  float* o_act, float* o_rew, float* o_nxt, float* o_mask, long long* o_idx, cudaStream_t st);
+// n-step returns (uavca_nstep.cuh): the slots of launch_replay_sample / launch_per_sample, then the n-step gather
+cudaError_t launch_replay_sample_nstep(const float* r_obs, const float* r_act, const float* r_rew, const float* r_nxt,
+                                       const float* r_mask, long long capacity, int obs_dim, int act_dim, const long long* meta,
+                                       long long batch, unsigned long long seed, unsigned long long draw, int recency,
+                                       long long stride, int n, double gamma, float* o_obs, float* o_act, float* o_rew,
+                                       float* o_nxt, float* o_disc, long long* o_idx, cudaStream_t st);
 
 // Prioritized replay (uavca_per.cu): the sum-tree over the ring's slots.
 cudaError_t launch_per_sync(double* tree, long long L, long long* per_meta, const long long* ring_meta, long long capacity,
@@ -42,6 +48,12 @@ cudaError_t launch_per_sample(const float* r_obs, const float* r_act, const floa
                               long long L, long long batch, double beta, unsigned long long seed, unsigned long long draw,
                               float* o_obs, float* o_act, float* o_rew, float* o_nxt, float* o_mask, long long* o_idx,
                               float* o_w, cudaStream_t st);
+cudaError_t launch_per_sample_nstep(const float* r_obs, const float* r_act, const float* r_rew, const float* r_nxt,
+                                    const float* r_mask, long long capacity, int obs_dim, int act_dim,
+                                    const long long* ring_meta, double* tree, long long L, long long batch, double beta,
+                                    long long stride, int n, double gamma, unsigned long long seed, unsigned long long draw,
+                                    float* o_obs, float* o_act, float* o_rew, float* o_nxt, float* o_disc, long long* o_idx,
+                                    float* o_w, cudaStream_t st);
 
 cudaError_t launch_policy_act(const float* obs, long long M, const void* w1, const void* w2, const void* w2b, const void* w3,
                               const void* w3b, const float* noise, unsigned long long seed, unsigned long long counter,

@@ -15,6 +15,7 @@
 #include "uavca_multi.cuh"
 #include "uavca_seq.cuh"
 #include "uavca_cta.cuh"
+#include "uavca_nstep.cuh"
 
 namespace uavca {
 
@@ -773,18 +774,13 @@ __global__ void __launch_bounds__(kPushThreads) replay_push_kernel(const V* obs,
 // sample, draw + appends so far) (uavca_device.cuh), so a learner step captured in a CUDA graph samples fresh transitions
 // from the ring as it grows.  An empty ring yields slot 0.
 // 16 threads per sample: they share the slot and copy the rows element-wise.
-constexpr int kSampleLanes = 16;
-__global__ void __launch_bounds__(kThreads) replay_sample_kernel(const float* r_obs, const float* r_act, const float* r_rew,
-                                                                 const float* r_nxt, const float* r_mask, long long cap, int od,
-                                                                 int ad, const long long* meta, long long batch, unsigned seed_lo,
-                                                                 unsigned seed_hi, unsigned long long draw, int recency,
-                                                                 float* o_obs, float* o_act, float* o_rew, float* o_nxt,
-                                                                 float* o_mask, long long* o_idx) {
-  const long long j = ((long long)blockIdx.x * kThreads + threadIdx.x) / kSampleLanes;
-  const int l = threadIdx.x % kSampleLanes;
-  if (j >= batch) return;
-  const long long head = meta[0], size = meta[2];
-  const unsigned long long ctr = draw + (unsigned long long)meta[3];
+constexpr int kSampleLanes = kNstepLanes;
+
+// The slot of sample j, drawn from the sampler's stream (tag 5) at counter ctr = draw + appends so far; shared by the
+// one-step and the n-step sampler, so that both draw the same slots for the same (seed, draw, appends).
+__device__ __forceinline__ long long replay_draw_slot(long long head, long long size, long long cap, long long j,
+                                                      unsigned long long ctr, unsigned seed_lo, unsigned seed_hi,
+                                                      int recency) {
   const uint4 r = philox_indexed(kStreamSample, (unsigned long long)j, ctr, seed_lo, seed_hi);
   long long slot = 0;
   if (size > 0) {
@@ -800,6 +796,21 @@ __global__ void __launch_bounds__(kThreads) replay_sample_kernel(const float* r_
       slot = (long long)(((unsigned long long)r.x * (unsigned long long)size) >> 32);  // uniform over the filled slots (size < 2^32)
     }
   }
+  return slot;
+}
+
+__global__ void __launch_bounds__(kThreads) replay_sample_kernel(const float* r_obs, const float* r_act, const float* r_rew,
+                                                                 const float* r_nxt, const float* r_mask, long long cap, int od,
+                                                                 int ad, const long long* meta, long long batch, unsigned seed_lo,
+                                                                 unsigned seed_hi, unsigned long long draw, int recency,
+                                                                 float* o_obs, float* o_act, float* o_rew, float* o_nxt,
+                                                                 float* o_mask, long long* o_idx) {
+  const long long j = ((long long)blockIdx.x * kThreads + threadIdx.x) / kSampleLanes;
+  const int l = threadIdx.x % kSampleLanes;
+  if (j >= batch) return;
+  const long long head = meta[0], size = meta[2];
+  const unsigned long long ctr = draw + (unsigned long long)meta[3];
+  const long long slot = replay_draw_slot(head, size, cap, j, ctr, seed_lo, seed_hi, recency);
   for (int k = l; k < od; k += kSampleLanes) {
     o_obs[j * od + k] = r_obs[slot * od + k];
     o_nxt[j * od + k] = r_nxt[slot * od + k];
@@ -810,6 +821,24 @@ __global__ void __launch_bounds__(kThreads) replay_sample_kernel(const float* r_
     o_mask[j] = r_mask[slot];
     if (o_idx) o_idx[j] = slot;
   }
+}
+
+// The n-step sampler: the same slots as replay_sample_kernel, then the n-step gather of uavca_nstep.cuh (include/uavca.h,
+// uavca_replay_sample_nstep).
+__global__ void __launch_bounds__(kThreads) replay_sample_nstep_kernel(
+    const float* r_obs, const float* r_act, const float* r_rew, const float* r_nxt, const float* r_mask, long long cap, int od,
+    int ad, const long long* meta, long long batch, unsigned seed_lo, unsigned seed_hi, unsigned long long draw, int recency,
+    long long stride, int n, double gamma, float* o_obs, float* o_act, float* o_rew, float* o_nxt, float* o_disc,
+    long long* o_idx) {
+  const long long j = ((long long)blockIdx.x * kThreads + threadIdx.x) / kSampleLanes;
+  const int l = threadIdx.x % kSampleLanes;
+  if (j >= batch) return;
+  const long long head = meta[0], size = meta[2];
+  const unsigned long long ctr = draw + (unsigned long long)meta[3];
+  const long long slot = replay_draw_slot(head, size, cap, j, ctr, seed_lo, seed_hi, recency);
+  nstep_gather(r_obs, r_act, r_rew, r_nxt, r_mask, od, ad, cap, head, stride, n, gamma, slot, j, l,
+               0xFFFFu << (threadIdx.x & 16), o_obs, o_act, o_rew, o_nxt, o_disc);
+  if (l == 0 && o_idx) o_idx[j] = slot;
 }
 
 // ================================================================================================================
@@ -987,6 +1016,18 @@ cudaError_t launch_replay_sample(const float* r_obs, const float* r_act, const f
   replay_sample_kernel<<<flat_grid(batch * kSampleLanes), kThreads, 0, st>>>(
       r_obs, r_act, r_rew, r_nxt, r_mask, capacity, obs_dim, act_dim, meta, batch, (unsigned)(seed & 0xffffffffull),
       (unsigned)(seed >> 32), draw, recency, o_obs, o_act, o_rew, o_nxt, o_mask, o_idx);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_replay_sample_nstep(const float* r_obs, const float* r_act, const float* r_rew, const float* r_nxt,
+                                       const float* r_mask, long long capacity, int obs_dim, int act_dim, const long long* meta,
+                                       long long batch, unsigned long long seed, unsigned long long draw, int recency,
+                                       long long stride, int n, double gamma, float* o_obs, float* o_act, float* o_rew,
+                                       float* o_nxt, float* o_disc, long long* o_idx, cudaStream_t st) {
+  if (batch <= 0) return cudaSuccess;
+  replay_sample_nstep_kernel<<<flat_grid(batch * kSampleLanes), kThreads, 0, st>>>(
+      r_obs, r_act, r_rew, r_nxt, r_mask, capacity, obs_dim, act_dim, meta, batch, (unsigned)(seed & 0xffffffffull),
+      (unsigned)(seed >> 32), draw, recency, stride, n, gamma, o_obs, o_act, o_rew, o_nxt, o_disc, o_idx);
   return cudaGetLastError();
 }
 

@@ -9,6 +9,7 @@
 #include <cfloat>
 
 #include "uavca_host.h"
+#include "uavca_nstep.cuh"
 
 namespace uavca {
 
@@ -18,7 +19,7 @@ constexpr int kSyncThreads = 512;
 constexpr int kSyncLeaves = 1024;      // leaves per CTA block of the sync kernel (2 per thread), reduced in shared memory
 constexpr int kUpdateThreads = 1024;   // the update is one CTA: its steps are separated by block barriers
 constexpr int kSampleThreads = 256;
-constexpr int kSampleLanes = 16;       // lanes per sample: one node each of a 4-level chunk of the descent, then the gather
+constexpr int kSampleLanes = kNstepLanes;  // lanes per sample: one node each of a 4-level chunk of the descent, then the gather
 constexpr unsigned long long kMark = 0xFFF0000000000000ull;  // bits of -inf: above it the leaf holds an update's marker
 
 __device__ __forceinline__ unsigned long long* ticket(double* tree) { return reinterpret_cast<unsigned long long*>(tree); }
@@ -214,11 +215,53 @@ __device__ __forceinline__ double pair_sum(double x, int d, int g, unsigned mask
   return (g & d) ? __dadd_rn(o, x) : __dadd_rn(x, o);  // left child first on both lanes
 }
 
+// The slot of sample j (the 16 lanes of its group: lane g, shuffle mask `mask`): stratified u on the prioritized stream
+// (tag 6) at counter draw + appends so far, then the descent; slot 0 when the tree is empty.  Shared by the one-step and
+// the n-step sampler, so that both draw the same slots for the same (seed, draw, appends, tree).
+__device__ __forceinline__ long long per_draw_slot(const double* tree, long long L, int D, double total, const long long* rm,
+                                                   long long j, long long batch, unsigned seed_lo, unsigned seed_hi,
+                                                   unsigned long long draw, int g, unsigned mask) {
+  long long slot = 0;
+  if (total > 0.0) {
+    const unsigned long long ctr = draw + (unsigned long long)rm[3];
+    const uint4 r = philox_indexed(kStreamPerSample, (unsigned long long)j, ctr, seed_lo, seed_hi);
+    double u = __dmul_rn(__ddiv_rn(__dadd_rn((double)j, u53(r.x, r.y)), (double)batch), total);
+    long long node = 1;
+    for (int left = D; left > 0;) {
+      const int lv = left < 4 ? left : 4;
+      const int width = 1 << lv;
+      const long long base = node << lv;
+      const double v = g < width ? tree[base + g] : 0.0;
+      const double s1 = pair_sum(v, 1, g, mask), s2 = pair_sum(s1, 2, g, mask), s3 = pair_sum(s2, 4, g, mask);
+      int pos = 0;
+      for (int w = width >> 1; w >= 1; w >>= 1) {
+        const double sw = w == 8 ? s3 : w == 4 ? s2 : w == 2 ? s1 : v;
+        const double lft = __shfl_sync(mask, sw, pos, kSampleLanes);
+        const double rgt = __shfl_sync(mask, sw, pos + w, kSampleLanes);
+        if (!(u < lft) && rgt != 0.0) {  // go left if u < left or the right subtree is empty
+          u = __dsub_rn(u, lft);
+          pos += w;
+        }
+      }
+      node = base + pos;
+      left -= lv;
+    }
+    slot = node - L;
+  }
+  return slot;
+}
+
+// One kernel for both samplers: kNstep = false is uavca_per_sample (the drawn rows and their mask), true is
+// uavca_per_sample_nstep (the n-step gather of uavca_nstep.cuh, its discount in o_mask; cap, stride, n and gamma are
+// read only there).  The weight pass stays in the kernel body: as a separate function it costs the one-step instance a
+// spilled pointer around the pow calls.  The last CTA to take a ticket (tree[0]) forms the weights, w_j = (size * P_j)^-beta
+// with P_j = leaf / total, divided by the largest w of the batch (batch < 2^26: int indices), and gives the ticket back.
+template <bool kNstep>
 __global__ void __launch_bounds__(kSampleThreads) per_sample_kernel(
-    const float* r_obs, const float* r_act, const float* r_rew, const float* r_nxt, const float* r_mask, int od, int ad,
-    const long long* rm, double* tree, long long L, int D, long long batch, double beta, unsigned seed_lo, unsigned seed_hi,
-    unsigned long long draw, float* o_obs, float* o_act, float* o_rew, float* o_nxt, float* o_mask, long long* o_idx,
-    float* o_w) {
+    const float* r_obs, const float* r_act, const float* r_rew, const float* r_nxt, const float* r_mask, long long cap, int od,
+    int ad, const long long* rm, double* tree, long long L, int D, long long batch, double beta, long long stride, int n,
+    double gamma, unsigned seed_lo, unsigned seed_hi, unsigned long long draw, float* o_obs, float* o_act, float* o_rew,
+    float* o_nxt, float* o_mask, long long* o_idx, float* o_w) {
   __shared__ bool last;
   __shared__ double red[kSampleThreads / 32];
   const long long j = ((long long)blockIdx.x * kSampleThreads + threadIdx.x) / kSampleLanes;
@@ -226,42 +269,22 @@ __global__ void __launch_bounds__(kSampleThreads) per_sample_kernel(
   const unsigned mask = 0xFFFFu << (threadIdx.x & 16);
   const double total = tree[1];
   if (j < batch) {
-    long long slot = 0;
-    if (total > 0.0) {
-      const unsigned long long ctr = draw + (unsigned long long)rm[3];
-      const uint4 r = philox_indexed(kStreamPerSample, (unsigned long long)j, ctr, seed_lo, seed_hi);
-      double u = __dmul_rn(__ddiv_rn(__dadd_rn((double)j, u53(r.x, r.y)), (double)batch), total);
-      long long node = 1;
-      for (int left = D; left > 0;) {
-        const int lv = left < 4 ? left : 4;
-        const int width = 1 << lv;
-        const long long base = node << lv;
-        const double v = g < width ? tree[base + g] : 0.0;
-        const double s1 = pair_sum(v, 1, g, mask), s2 = pair_sum(s1, 2, g, mask), s3 = pair_sum(s2, 4, g, mask);
-        int pos = 0;
-        for (int w = width >> 1; w >= 1; w >>= 1) {
-          const double sw = w == 8 ? s3 : w == 4 ? s2 : w == 2 ? s1 : v;
-          const double lft = __shfl_sync(mask, sw, pos, kSampleLanes);
-          const double rgt = __shfl_sync(mask, sw, pos + w, kSampleLanes);
-          if (!(u < lft) && rgt != 0.0) {  // go left if u < left or the right subtree is empty
-            u = __dsub_rn(u, lft);
-            pos += w;
-          }
-        }
-        node = base + pos;
-        left -= lv;
+    const long long slot = per_draw_slot(tree, L, D, total, rm, j, batch, seed_lo, seed_hi, draw, g, mask);
+    if constexpr (kNstep) {
+      nstep_gather(r_obs, r_act, r_rew, r_nxt, r_mask, od, ad, cap, rm[0], stride, n, gamma, slot, j, g, mask, o_obs, o_act,
+                   o_rew, o_nxt, o_mask);
+      if (g == 0) o_idx[j] = slot;
+    } else {
+      for (int k = g; k < od; k += kSampleLanes) {
+        o_obs[j * od + k] = r_obs[slot * od + k];
+        o_nxt[j * od + k] = r_nxt[slot * od + k];
       }
-      slot = node - L;
-    }
-    for (int k = g; k < od; k += kSampleLanes) {
-      o_obs[j * od + k] = r_obs[slot * od + k];
-      o_nxt[j * od + k] = r_nxt[slot * od + k];
-    }
-    for (int k = g; k < ad; k += kSampleLanes) o_act[j * ad + k] = r_act[slot * ad + k];
-    if (g == 0) {
-      o_rew[j] = r_rew[slot];
-      o_mask[j] = r_mask[slot];
-      o_idx[j] = slot;
+      for (int k = g; k < ad; k += kSampleLanes) o_act[j * ad + k] = r_act[slot * ad + k];
+      if (g == 0) {
+        o_rew[j] = r_rew[slot];
+        o_mask[j] = r_mask[slot];
+        o_idx[j] = slot;
+      }
     }
   }
   __syncthreads();
@@ -272,7 +295,6 @@ __global__ void __launch_bounds__(kSampleThreads) per_sample_kernel(
   __syncthreads();
   if (!last) return;
   __threadfence();
-  // w_j = (size * P_j)^-beta with P_j = leaf / total, divided by the largest w of the batch (batch < 2^26: int indices)
   const double size = (double)rm[2];
   const double* leaf = tree + L;
   const int nb = (int)batch;
@@ -334,10 +356,24 @@ cudaError_t launch_per_sample(const float* r_obs, const float* r_act, const floa
                               float* o_w, cudaStream_t st) {
   if (batch <= 0) return cudaSuccess;
   const long long grid = (batch * kSampleLanes + kSampleThreads - 1) / kSampleThreads;
-  per_sample_kernel<<<(int)grid, kSampleThreads, 0, st>>>(r_obs, r_act, r_rew, r_nxt, r_mask, obs_dim, act_dim, ring_meta,
-                                                         tree, L, log2_exact(L), batch, beta, (unsigned)(seed & 0xffffffffull),
-                                                         (unsigned)(seed >> 32), draw, o_obs, o_act, o_rew, o_nxt, o_mask,
-                                                         o_idx, o_w);
+  per_sample_kernel<false><<<(int)grid, kSampleThreads, 0, st>>>(
+      r_obs, r_act, r_rew, r_nxt, r_mask, 0, obs_dim, act_dim, ring_meta, tree, L, log2_exact(L), batch, beta, 0, 1, 0.0,
+      (unsigned)(seed & 0xffffffffull), (unsigned)(seed >> 32), draw, o_obs, o_act, o_rew, o_nxt, o_mask, o_idx, o_w);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_per_sample_nstep(const float* r_obs, const float* r_act, const float* r_rew, const float* r_nxt,
+                                    const float* r_mask, long long capacity, int obs_dim, int act_dim,
+                                    const long long* ring_meta, double* tree, long long L, long long batch, double beta,
+                                    long long stride, int n, double gamma, unsigned long long seed, unsigned long long draw,
+                                    float* o_obs, float* o_act, float* o_rew, float* o_nxt, float* o_disc, long long* o_idx,
+                                    float* o_w, cudaStream_t st) {
+  if (batch <= 0) return cudaSuccess;
+  const long long grid = (batch * kSampleLanes + kSampleThreads - 1) / kSampleThreads;
+  per_sample_kernel<true><<<(int)grid, kSampleThreads, 0, st>>>(
+      r_obs, r_act, r_rew, r_nxt, r_mask, capacity, obs_dim, act_dim, ring_meta, tree, L, log2_exact(L), batch, beta, stride,
+      n, gamma, (unsigned)(seed & 0xffffffffull), (unsigned)(seed >> 32), draw, o_obs, o_act, o_rew, o_nxt, o_disc, o_idx,
+      o_w);
   return cudaGetLastError();
 }
 

@@ -155,6 +155,27 @@ def replay_sample(ring_obs: torch.Tensor, ring_action: torch.Tensor, ring_reward
                                                  _ptr(out_index), _stream(ring_obs)), "uavca_replay_sample")
 
 
+@torch.library.custom_op("uavca::replay_sample_nstep",
+                         mutates_args=("out_obs", "out_action", "out_reward", "out_next_obs", "out_discount", "out_index"))
+def replay_sample_nstep(ring_obs: torch.Tensor, ring_action: torch.Tensor, ring_reward: torch.Tensor,
+                        ring_next_obs: torch.Tensor, ring_mask: torch.Tensor, ring_meta: torch.Tensor, seed: int, draw: int,
+                        recency_weighted: bool, stride: int, n: int, gamma: float, out_obs: torch.Tensor,
+                        out_action: torch.Tensor, out_reward: torch.Tensor, out_next_obs: torch.Tensor,
+                        out_discount: torch.Tensor, out_index: Optional[torch.Tensor]) -> None:
+    """The slots of `replay_sample` with n-step returns folded over up to `n` successors `stride` slots apart, in one
+    launch (rule in include/uavca.h, uavca_replay_sample_nstep)."""
+    _need_cuda(ring_obs, ring_action, ring_reward, ring_next_obs, ring_mask, ring_meta, out_obs, out_action, out_reward,
+               out_next_obs, out_discount, out_index)
+    cap, batch = ring_reward.numel(), out_reward.numel()
+    _capi.check(_capi.load().uavca_replay_sample_nstep(ring_obs.data_ptr(), ring_action.data_ptr(), ring_reward.data_ptr(),
+                                                       ring_next_obs.data_ptr(), ring_mask.data_ptr(), cap,
+                                                       ring_obs.numel() // cap, ring_action.numel() // cap,
+                                                       ring_meta.data_ptr(), batch, seed, draw, int(recency_weighted),
+                                                       stride, n, float(gamma), out_obs.data_ptr(), out_action.data_ptr(),
+                                                       out_reward.data_ptr(), out_next_obs.data_ptr(), out_discount.data_ptr(),
+                                                       _ptr(out_index), _stream(ring_obs)), "uavca_replay_sample_nstep")
+
+
 def _per_tree(tree: torch.Tensor, per_meta: Optional[torch.Tensor]) -> int:
     """Checks the sum-tree and per_meta tensors of prioritized replay; returns L."""
     if tree.dtype != torch.float64 or tree.dim() != 1 or tree.numel() < 2 or tree.numel() % 2:
@@ -206,6 +227,32 @@ def per_sample(ring_obs: torch.Tensor, ring_action: torch.Tensor, ring_reward: t
                                               float(beta), seed, draw, out_obs.data_ptr(), out_action.data_ptr(),
                                               out_reward.data_ptr(), out_next_obs.data_ptr(), out_mask.data_ptr(),
                                               out_index.data_ptr(), out_weight.data_ptr(), _stream(tree)), "uavca_per_sample")
+
+
+@torch.library.custom_op("uavca::per_sample_nstep", mutates_args=("tree", "out_obs", "out_action", "out_reward",
+                                                                 "out_next_obs", "out_discount", "out_index", "out_weight"))
+def per_sample_nstep(ring_obs: torch.Tensor, ring_action: torch.Tensor, ring_reward: torch.Tensor,
+                     ring_next_obs: torch.Tensor, ring_mask: torch.Tensor, ring_meta: torch.Tensor, tree: torch.Tensor,
+                     batch: int, beta: float, stride: int, n: int, gamma: float, seed: int, draw: int,
+                     out_obs: torch.Tensor, out_action: torch.Tensor, out_reward: torch.Tensor, out_next_obs: torch.Tensor,
+                     out_discount: torch.Tensor, out_index: torch.Tensor, out_weight: torch.Tensor) -> None:
+    """The slots and weights of `per_sample` with n-step returns (include/uavca.h, uavca_per_sample_nstep), one launch.
+    (`tree` is listed as mutated: its element 0 is the launch's CTA ticket.)"""
+    _need_cuda(ring_obs, ring_action, ring_reward, ring_next_obs, ring_mask, ring_meta, tree, out_obs, out_action,
+               out_reward, out_next_obs, out_discount, out_index, out_weight)
+    L = _per_tree(tree, None)
+    if out_index.dtype != torch.int64 or out_weight.dtype != torch.float32 or out_index.numel() != batch or \
+            out_weight.numel() != batch or out_reward.numel() != batch:
+        raise _capi.UavcaError("per_sample_nstep: out_index int64 [batch], out_weight float32 [batch]")
+    cap = ring_reward.numel()
+    _capi.check(_capi.load().uavca_per_sample_nstep(ring_obs.data_ptr(), ring_action.data_ptr(), ring_reward.data_ptr(),
+                                                    ring_next_obs.data_ptr(), ring_mask.data_ptr(), cap,
+                                                    ring_obs.numel() // cap, ring_action.numel() // cap,
+                                                    ring_meta.data_ptr(), tree.data_ptr(), L, batch, float(beta), stride, n,
+                                                    float(gamma), seed, draw, out_obs.data_ptr(), out_action.data_ptr(),
+                                                    out_reward.data_ptr(), out_next_obs.data_ptr(), out_discount.data_ptr(),
+                                                    out_index.data_ptr(), out_weight.data_ptr(), _stream(tree)),
+                "uavca_per_sample_nstep")
 
 
 @torch.library.custom_op("uavca::step_multi_replay",

@@ -81,6 +81,30 @@ class DeviceReplay:
         self._draws += 1
         return out
 
+    def sample_nstep(self, batch_size: int, n: int, gamma: float, stride: int, recency_weighted: bool = False, out=None,
+                     want_index: bool = False):
+        """`sample_fused` with n-step returns, in ONE launch with no host synchronisation (`uavca_replay_sample_nstep`):
+        the same slots as `sample_fused` at the same draw count, then up to n - 1 successors `stride` slots apart
+        (stride = envs * agents of the multi world, envs of the single world) are folded while they continue the
+        episode.  Returns (state, action, reward_n, next_state_n, discount[, index]); the learner's target is
+        reward_n + discount * V(next_state_n), which for n = 1 is r + gamma * mask * V.  The episode rule (include/uavca.h):
+        a successor chains when the ring's mask is 1 and its observation equals the previous next observation bit for bit,
+        so auto-resets, terminal transitions and the newest slots all end the return early with the matching gamma^k.
+        Checked before the launch: 1 <= n <= 16, 1 <= stride <= capacity, 0 <= gamma <= 1.  Advances the draw count
+        of `sample_fused`."""
+        if out is None:
+            kw = dict(dtype=torch.float32, device=self.device)
+            out = (torch.empty((batch_size, self.obs_dim), **kw), torch.empty((batch_size, self.act_dim), **kw),
+                   torch.empty(batch_size, **kw), torch.empty((batch_size, self.obs_dim), **kw), torch.empty(batch_size, **kw))
+            if want_index:
+                out = out + (torch.empty(batch_size, dtype=torch.int64, device=self.device),)
+        idx = out[5] if len(out) > 5 else None
+        ops.replay_sample_nstep(self.state, self.action, self.reward, self.next_state, self.mask, self.meta,
+                                self._sample_seed, self._draws, bool(recency_weighted), int(stride), int(n), float(gamma),
+                                out[0], out[1], out[2], out[3], out[4], idx)
+        self._draws += 1
+        return out
+
     def sample(self, batch_size: int, recency_weighted: bool = False):
         """-> (state [b,obs], action [b,act], reward [b], next_state [b,obs], mask [b]) as `memory.sample` returns them
         (pytorch_sac_temp/sac.py:48).  Uniform with replacement, or with probability rising linearly with recency
@@ -151,6 +175,22 @@ class PrioritizedDeviceReplay(DeviceReplay):
                    torch.empty(batch_size, dtype=torch.int64, device=self.device), torch.empty(batch_size, **kw))
         ops.per_sample(self.state, self.action, self.reward, self.next_state, self.mask, self.meta, self.tree, batch_size,
                        float(beta), self._sample_seed, self._per_draws, *out)
+        self._per_draws += 1
+        return out
+
+    def sample_prioritized_nstep(self, batch_size: int, beta: float, n: int, gamma: float, stride: int, out=None):
+        """`sample_prioritized` with the n-step returns of `DeviceReplay.sample_nstep`, in ONE launch: -> (state, action,
+        reward_n, next_state_n, discount, index int64, weight float32).  The same slots and weights as
+        `sample_prioritized` at the same draw count; write the n-step TD error of `index` back with `update_priorities`
+        (the Ape-X learner).  Advances the draw count of `sample_prioritized`."""
+        if out is None:
+            kw = dict(dtype=torch.float32, device=self.device)
+            out = (torch.empty((batch_size, self.obs_dim), **kw), torch.empty((batch_size, self.act_dim), **kw),
+                   torch.empty(batch_size, **kw), torch.empty((batch_size, self.obs_dim), **kw), torch.empty(batch_size, **kw),
+                   torch.empty(batch_size, dtype=torch.int64, device=self.device), torch.empty(batch_size, **kw))
+        ops.per_sample_nstep(self.state, self.action, self.reward, self.next_state, self.mask, self.meta, self.tree,
+                             batch_size, float(beta), int(stride), int(n), float(gamma), self._sample_seed, self._per_draws,
+                             *out)
         self._per_draws += 1
         return out
 

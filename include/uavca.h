@@ -17,6 +17,7 @@
  *   uavca_replay_push(_dev) / uavca_replay_sample <- ReplayMemory.push / .sample   pytorch_sac_temp/replay_memory.py:15-24
  *   uavca_per_sync / uavca_per_update / uavca_per_sample <- no reference counterpart: prioritized replay over the device ring
  *                         (Schaul et al. 2016, the sum-tree of the Ape-X learner, Horgan et al. 2018)
+ *   uavca_replay_sample_nstep / uavca_per_sample_nstep <- no reference counterpart: n-step returns from the device ring
  *   uavca_stats        <- env.steps / target_reach_count / collision_count  multi_uav_world_2d.py:166-168,209,221,238
  *   uavca_config       <- constructor kwargs              multi_uav_world_2d.py:13-28, uav_world_2d.py:14-26
  *
@@ -37,7 +38,7 @@
 extern "C" {
 #endif
 
-#define UAVCA_VERSION 204
+#define UAVCA_VERSION 205
 
 /* world kinds */
 #define UAVCA_KIND_MULTI 0  /* MultiUAVWorld2D: N UAVs per env, 10-feature observation */
@@ -296,6 +297,52 @@ int uavca_per_sample(const float* ring_obs, const float* ring_action, const floa
                      double* tree, int64_t L, int64_t batch, double beta, uint64_t seed, uint64_t draw, float* out_obs,
                      float* out_action, float* out_reward, float* out_next_obs, float* out_mask, int64_t* out_index,
                      float* out_weight, void* stream);
+
+/* n-step returns (Ape-X, Horgan et al. 2018; Rainbow; R2D2): R = sum_{i<k} gamma^i r_{t+i}, bootstrapped with
+ * gamma^k Q(s_{t+k}, .), for the slots of uavca_replay_sample / uavca_per_sample, in ONE launch each.
+ *
+ * Appends of `stride` transitions per acting step put UAV m of step t at slot (head_t + m) mod capacity, on both append
+ * paths (uavca_step_multi_replay, uavca_replay_push_dev), so the successor of slot s is s_i = (s + i * stride) mod capacity;
+ * stride is B * N for the multi world and B for the single world.  For a drawn slot s_0 = s:
+ *   age(s) = (ring_meta[0] - 1 - s) mod capacity (the newest slot has age 0);
+ *   link i (1 <= i < n) holds iff ring_mask[s_{i-1}] != 0, i * stride <= age(s) (s_i was appended after s and has not
+ *     been overwritten), and ring_obs[s_i] equals ring_next_obs[s_{i-1}] bit for bit over all obs_dim floats;
+ *   k = 1 + the number of links that hold consecutively from i = 1, so 1 <= k <= n;
+ *   R: in float64, sequential and unfused, g = 1, R = 0; for i < k: R = R + g * r_i; g = g * gamma; rounded once to float;
+ *   discount = float(g) (gamma^k as that product) if ring_mask[s_{k-1}] != 0, else 0.
+ * Outputs: out_obs = ring_obs[s], out_action = ring_action[s], out_reward = R, out_next_obs = ring_next_obs[s_{k-1}],
+ * out_discount, out_index = s.  The learner's target is R + discount * V(next_obs); for n = 1 it is exactly today's
+ * r + gamma * mask * V (out_discount = float(gamma) * mask).
+ *
+ * The third condition is the episode test.  A transition chains into the next one exactly when the next one was acted on
+ * from the observation this one ended in: without an auto-reset the step writes obs and final_obs / ring next_obs from
+ * the same rows, after one the acted-on observation is the post-reset one.  A wrong stride, appends of mixed sizes or a
+ * slot overwritten by a wrap fail the test too and give shorter returns, never wrong ones.  The one limitation: a
+ * post-reset observation equal bit for bit to the pre-reset one (an identical reset state and an unmoved UAV) is chained.
+ * The newest (n - 1) * stride slots yield truncated returns (k < n) with the matching gamma^k; they are not excluded, so
+ * each sampler's slot law stays exactly its one-step law.
+ *
+ * The slots are those of the one-step sibling: the same Philox stream (tag 5, tag 6), counters and draw code, so for the
+ * same (seed, draw, appends) the n-step call draws the same slots.  Host arguments, checked before the launch:
+ * 1 <= n <= 16, 1 <= stride <= capacity, 0 <= gamma <= 1.  An empty ring yields slot 0, whose rows are zeros, with
+ * discount 0 (its mask is 0).  No host synchronisation: safe inside a CUDA graph of a learner step, which draws afresh as
+ * appends advance ring_meta[3]. */
+int uavca_replay_sample_nstep(const float* ring_obs, const float* ring_action, const float* ring_reward,
+                              const float* ring_next_obs, const float* ring_mask, int64_t capacity, int32_t obs_dim,
+                              int32_t act_dim, const int64_t* ring_meta, int64_t batch, uint64_t seed, uint64_t draw,
+                              int recency_weighted, int64_t stride, int32_t n, double gamma, float* out_obs,
+                              float* out_action, float* out_reward, float* out_next_obs, float* out_discount,
+                              int64_t* out_index, void* stream);
+
+/* uavca_per_sample with the n-step gather above: the same slots, out_index and importance weights (the prioritized
+ * stream, tag 6); out_discount in place of out_mask.  The learner writes the n-step TD error of slot out_index back with
+ * uavca_per_update, as the Ape-X learner does. */
+int uavca_per_sample_nstep(const float* ring_obs, const float* ring_action, const float* ring_reward,
+                           const float* ring_next_obs, const float* ring_mask, int64_t capacity, int32_t obs_dim,
+                           int32_t act_dim, const int64_t* ring_meta, double* tree, int64_t L, int64_t batch, double beta,
+                           int64_t stride, int32_t n, double gamma, uint64_t seed, uint64_t draw, float* out_obs,
+                           float* out_action, float* out_reward, float* out_next_obs, float* out_discount,
+                           int64_t* out_index, float* out_weight, void* stream);
 
 /* uavca_step_multi with the replay append folded into the SAME launch ("next" row; MultiUAVWorld2D.step followed by the N
  * memory.push calls of test_sac_multi.py:99-103).  Besides everything uavca_step_multi writes, UAV m's transition goes to

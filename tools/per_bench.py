@@ -1,6 +1,7 @@
 """Prioritized replay on one GPU: sum-tree sync, priority update and prioritized sampling against the PyTorch ways of
-drawing from a priority vector, and what the sync adds to the configs[4] acting step.  CUDA events; ring of 1,048,576
-slots (2^20 leaves).
+drawing from a priority vector, what the sync adds to the configs[4] acting step, and the n-step samplers against the
+one-step draws and against the same n-step rule written with torch indexing.  CUDA events; ring of 1,048,576 slots
+(2^20 leaves).
     python tools/per_bench.py [--reps N]"""
 import argparse
 import json
@@ -51,6 +52,65 @@ def graph_us(fn, n=20, reps=5):
         e1.record(st)
     st.synchronize()
     return e0.elapsed_time(e1) * 1e3 / (reps * n)
+
+
+def torch_nstep(rb, idx, n, gamma, stride):
+    """The n-step rule of include/uavca.h (uavca_replay_sample_nstep) for slots `idx`, written with torch indexing: what a
+    learner would run without the fused sampler.  No host synchronisation, so it can be captured too."""
+    cap = rb.capacity
+    age = torch.remainder(rb.meta[0] - 1 - idx, cap)
+    ob, nb = rb.state.view(torch.int32), rb.next_state.view(torch.int32)
+    k = torch.ones_like(idx)
+    alive = torch.ones_like(idx, dtype=torch.bool)
+    prev = idx
+    for i in range(1, n):
+        si = torch.remainder(idx + i * stride, cap)
+        alive = alive & (rb.mask[prev] != 0) & (age >= i * stride) & (ob[si] == nb[prev]).all(1)
+        k = k + alive
+        prev = si
+    R = torch.zeros(idx.shape, dtype=torch.float64, device=idx.device)
+    g = torch.ones_like(R)
+    for i in range(n):
+        on = k > i
+        R = torch.where(on, R + g * rb.reward[torch.remainder(idx + i * stride, cap)].double(), R)
+        g = torch.where(on, g * gamma, g)
+    last = torch.remainder(idx + (k - 1) * stride, cap)
+    disc = torch.where(rb.mask[last] != 0, g.float(), torch.zeros_like(rb.mask[last]))
+    return rb.state[idx], rb.action[idx], R.float(), rb.next_state[last], disc
+
+
+def nstep_rows(res):
+    """The n-step samplers on a 2^20-slot prioritized ring filled by configs[4] acting steps (fused append + sync)."""
+    env = G.BatchedMultiUAVWorld2D(B4, num_agents=N4, reset_mode=G.RESET_ON_DONE0, max_episode_steps=100, seed=3)
+    rb = G.PrioritizedDeviceReplay(CAP, 10, 2, seed=0)
+    ro = G.BatchedRollout(env, None, rb, action_mode="polar", warmup_uniform=True)
+    ro.reset()
+    ro.run(8)  # 8 x 163,840 transitions: the ring is full and has wrapped
+    stride, gamma = B4 * N4, 0.99
+    for b in (256, 4096):
+        uni = rb.sample_fused(b, want_index=True)
+        res[f"nstep_sample_fused_{b}_us"] = graph_us(lambda: rb.sample_fused(b, out=uni))
+        per = rb.sample_prioritized(b, 0.4)
+        res[f"nstep_sample_prioritized_{b}_us"] = graph_us(lambda: rb.sample_prioritized(b, 0.4, out=per))
+        for n in (1, 3, 5):
+            un = rb.sample_nstep(b, n, gamma, stride, want_index=True)
+            res[f"sample_nstep_n{n}_{b}_us"] = graph_us(lambda: rb.sample_nstep(b, n, gamma, stride, out=un))
+            pn = rb.sample_prioritized_nstep(b, 0.4, n, gamma, stride)
+            res[f"sample_prioritized_nstep_n{n}_{b}_us"] = graph_us(
+                lambda: rb.sample_prioritized_nstep(b, 0.4, n, gamma, stride, out=pn))
+
+            def torch_rule():
+                rb.sample_fused(b, out=uni)
+                return torch_nstep(rb, uni[5], n, gamma, stride)
+
+            res[f"torch_nstep_n{n}_{b}_us"] = graph_us(torch_rule)
+    # the fused sampler and the torch rule agree on the same slots
+    d0 = rb._draws
+    got = rb.sample_nstep(4096, 3, gamma, stride, want_index=True)
+    rb._draws = d0
+    ref = torch_nstep(rb, rb.sample_fused(4096, want_index=True)[5], 3, gamma, stride)
+    res["nstep_torch_rule_agrees"] = all(torch.equal(x, y) for x, y in zip(got[:5], ref))
+    del env, rb, ro
 
 
 def main():
@@ -111,6 +171,7 @@ def main():
         res[f"acting_step_{kind}_us"] = graph_us(lambda: ro.run(2), n=10) / 2
         del env, ring, ro
     res["acting_step_sync_overhead_us"] = res["acting_step_prioritized_us"] - res["acting_step_uniform_us"]
+    nstep_rows(res)
     print(json.dumps(res))
 
 
